@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/s of the QuadX hover step (physics + reward + obs) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (QuadXHoverEnv.step for every env: 12
 physics sub-steps, 6 control updates, reward, termination, auto-reset, obs)
@@ -21,6 +21,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (it may be read-only)
 
 ALG_BYTES_PER_ENV_STEP = 358  # SURVEY 8d: 128+128 state, 16 action, 80 obs, 4 reward, 2 flags
 ACT_BYTES, OUT_BYTES, OUT_BYTES_BF16 = 16, 80 + 4 + 1 + 1, 40 + 4 + 1 + 1
@@ -41,7 +42,26 @@ def parse():
     ap.add_argument("--no-small", action="store_true", help="skip the configs[1] (4096 envs) side measurements")
     ap.add_argument("--no-ppo", action="store_true", help="skip the PPO rollout side measurements (metric M2)")
     ap.add_argument("--no-train", action="store_true", help="skip the bounded PPO training-to-target leg (SURVEY C5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (obs, reward, terminated, truncated, "
+                    "as float32; a fixed sample of DUMP_ENVS envs when there are more) to DIR/<name>.npy, rank 0's shard")
     return ap.parse_args()
+
+
+DUMP_ENVS = 1 << 18  # 262 144 envs x (20 + 3) float32 + the float64 env index = 26 MB per dump
+
+
+def last_step_outputs(obs, rew, te, tr) -> dict:
+    """The timed step's outputs for --dump-outputs, as host float32 arrays: every env, or above DUMP_ENVS a sample whose
+    indices depend only on the batch size, so that two builds run with the same arguments can be compared array by array."""
+    import numpy as np
+    import torch
+
+    n = obs.shape[0]
+    idx = np.sort(np.random.default_rng(0).choice(n, DUMP_ENVS, replace=False)) if n > DUMP_ENVS else np.arange(n)
+    i = torch.as_tensor(idx, device=obs.device)
+    out = {name: t[i].float().cpu().numpy() for name, t in (("obs", obs), ("reward", rew), ("terminated", te), ("truncated", tr))}
+    out["env_index"] = idx.astype(np.float64)
+    return out
 
 
 def workload_config(envs_per_gpu: int, n_gpus: int) -> dict:
@@ -370,6 +390,7 @@ def main_ours(args):
     ev1.record()
     torch.cuda.synchronize()
     t1 = time.perf_counter()
+    dump = last_step_outputs(obs, rew, te, tr) if args.dump_outputs and rank == 0 else None  # before the passes below overwrite them
     if world > 1:
         dist.barrier()
     launches = _lib.lib().qx_launch_count() - launches0
@@ -534,6 +555,10 @@ def main_ours(args):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if rank == 0:
         print(json.dumps(line))
 

@@ -1,5 +1,5 @@
-import sys, ctypes as C, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, ctypes as C, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import __graft_entry__ as ge; ge.build()
 from fpv_drone_rl_agent_b200 import _lib
 L = C.CDLL(_lib.LIB_PATH)

@@ -1,5 +1,5 @@
-import sys, statistics, torch
-sys.path.insert(0, '/root/repo')
+import os, sys, statistics, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import __graft_entry__ as ge; ge.build()
 from fpv_drone_rl_agent_b200 import ppo
 dev = torch.device('cuda')
