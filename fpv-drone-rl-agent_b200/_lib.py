@@ -13,6 +13,7 @@ LIB_PATH = os.environ.get("QX_LIB") or os.path.join(_HERE, "csrc", "libquadx_b20
 
 QX_TASK_HOVER, QX_TASK_YAW = 0, 1
 QX_OBS_F32, QX_OBS_BF16 = 0, 1
+QX_FRAME_RGBA, QX_FRAME_MASK = 0, 1
 QX_STATE_WORDS = 44
 QX_STATE_WORDS_CASCADE = 68
 
@@ -89,6 +90,7 @@ def lib() -> C.CDLL:
         "qx_step_end": (C.c_int, [vp, vp, i32, i64, vp]),
         "qx_done_queue": (C.c_int, [vp, C.POINTER(vp), C.POINTER(vp)]),
         "qx_step_k": (C.c_int, [vp, i32, f32p, f32p, f32p, u8p, u8p, vp]),
+        "qx_render": (C.c_int, [vp, vp, i64, i32, u8p, vp]),
         "qx_reset_host": (C.c_int, [vp, u8p, f32p]),
         "qx_step_host": (C.c_int, [vp, f32p, f32p, f32p, u8p, u8p, f32p]),
         "qx_step_host_ex": (C.c_int, [vp, f32p, vp, i32, f32p, u8p, u8p, f32p]),
@@ -142,7 +144,7 @@ def lib() -> C.CDLL:
 
 
 EXPORTED = [
-    "qx_default_config", "qx_create", "qx_destroy", "qx_reset", "qx_step", "qx_step_begin", "qx_step_end", "qx_done_queue", "qx_step_k", "qx_reset_host", "qx_step_host", "qx_step_host_ex",
+    "qx_default_config", "qx_create", "qx_destroy", "qx_reset", "qx_step", "qx_step_begin", "qx_step_end", "qx_done_queue", "qx_step_k", "qx_render", "qx_reset_host", "qx_step_host", "qx_step_host_ex",
     "qx_get_state", "qx_set_state", "qx_get_flags", "qx_episode_stats", "qx_nonfinite_count", "qx_num_envs", "qx_obs_dim", "qx_act_dim", "qx_state_ptr", "qx_state_words", "qx_uses_reference_constants", "qx_config_matches_reference_constants",
     "qx_launch_count", "qx_sizeof_config", "qx_last_error", "qx_version",
 ]

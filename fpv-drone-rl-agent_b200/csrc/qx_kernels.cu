@@ -878,6 +878,120 @@ __global__ void clock_probe_kernel(unsigned long long* out) {
   out[1] = ns;
 }
 
+// ---------------------------------------------------------------------------
+// K6: the FPV camera frame (qx_render).  One warp per 32-row band of a frame: lane l finds the covered columns of row
+// band * 32 + l with the helpers vision_raster uses, so a frame holds exactly the pixels vision_mode = 1 counts; then the
+// warp writes the band -- contiguous bytes of the frame -- with 16-byte stores, 512 contiguous bytes per store instruction.
+// ---------------------------------------------------------------------------
+constexpr int kRenderBlock = 256;
+constexpr uint32_t kRgbaBox = 0xFF0000C8u, kRgbaSky = 0xFFE6BEAAu;  // (200, 0, 0, 255) and (170, 190, 230, 255), little-endian RGBA
+struct RenderArgs {
+  const float4* state;
+  int64_t n;
+  const int32_t* env_idx;  // nullable: frame f shows env f
+  int64_t m;
+  uint8_t* frames;
+  int32_t res;
+  const float* raster;     // RasterConsts
+};
+
+// The box crosses the near plane (vision_raster reports it unseen; a yawed drone can still have part of it in view): the
+// silhouette is the projection of the box clipped to depth > cam_near, i.e. the convex hull of the corners in front and of the
+// points where edges cross the plane.  Those points go to the warp's slice of shared memory (every lane computes the same);
+// the hull's x interval on the row's centre line is the min / max over the vertex pairs crossing it (every such segment lies
+// inside the hull and every hull edge is one of them).  Rare, so kept out of registers.
+QX_DI void clipped_row_span(const RasterConsts& c, const float (&pxs)[8], const float (&pys)[8], const float (&xrs)[8], const float (&yus)[8],
+                            const float (&deps)[8], float2* __restrict__ pts, const int row, int& ln, int& rn) {
+  constexpr int ea[12] = {0, 1, 2, 3, 4, 5, 6, 7, 0, 1, 2, 3}, eb[12] = {1, 2, 3, 0, 5, 6, 7, 4, 4, 5, 6, 7};
+  const int lane = threadIdx.x & 31;
+  int nv = 0;
+#pragma unroll
+  for (int k = 0; k < 8; ++k)
+    if (deps[k] > c.cam_near) {
+      if (lane == 0) pts[nv] = make_float2(pxs[k], pys[k]);
+      ++nv;
+    }
+  const float k1 = c.inv_tan / c.cam_near;
+#pragma unroll
+  for (int e = 0; e < 12; ++e) {
+    const int a = ea[e], b = eb[e];
+    if ((deps[a] > c.cam_near) != (deps[b] > c.cam_near)) {
+      const float t = (c.cam_near - deps[a]) / (deps[b] - deps[a]);
+      const float xr = fmaf(t, xrs[b] - xrs[a], xrs[a]), yu = fmaf(t, yus[b] - yus[a], yus[a]);
+      if (lane == 0) pts[nv] = make_float2(fmaf(xr * k1, c.half_res, c.half_res), fmaf(-yu * k1, c.half_res, c.half_res));
+      ++nv;
+    }
+  }
+  __syncwarp();
+  ln = 1; rn = 0;
+  const float yl = (float)row + 0.5f;
+  float xl = 3.0e38f, xr = -3.0e38f;
+  for (int i = 1; i < nv; ++i) {
+    const float2 p = pts[i];
+    for (int j = 0; j < i; ++j) {
+      const float2 q = pts[j];
+      if ((p.y - yl) * (q.y - yl) <= 0.f && p.y != q.y) {
+        const float xi = fmaf(yl - p.y, (q.x - p.x) / (q.y - p.y), p.x);
+        xl = fminf(xl, xi); xr = fmaxf(xr, xi);
+      }
+    }
+  }
+  if (xl <= xr) { ln = (int)ceilf(xl - 0.5f); rn = (int)floorf(xr - 0.5f); }
+}
+
+// bits lo..hi (0 <= lo, hi <= 31) of a word; 0 when lo > hi
+QX_DI uint32_t run_bits(int lo, int hi) { return lo > hi ? 0u : (0xFFFFFFFFu >> (31 - (hi - lo))) << lo; }
+
+template <int FMT>
+__global__ void __launch_bounds__(kRenderBlock) render_kernel(const __grid_constant__ RenderArgs a) {
+  __shared__ float2 s_pts[kRenderBlock / 32][20];
+  constexpr int C = FMT == QX_FRAME_RGBA ? 4 : 1, PPC = 16 / C;  // bytes per pixel, pixels per 16-byte chunk
+  const int lane = threadIdx.x & 31, res = a.res, bands = (res + 31) >> 5;
+  const int64_t warp = ((int64_t)blockIdx.x * kRenderBlock + threadIdx.x) >> 5;
+  const int64_t f = warp / bands;
+  if (f >= a.m) return;  // whole warps
+  const int band = (int)(warp - f * bands);
+  const int64_t i = a.env_idx ? (int64_t)a.env_idx[f] : f;
+  int ln = 1, rn = 0;  // covered columns of row band * 32 + lane
+  if (i >= 0 && i < a.n) {
+    const RasterConsts c = *reinterpret_cast<const RasterConsts*>(a.raster);
+    const float4 p0 = a.state[i], p1 = a.state[a.n + i];  // (px py pz qx) (qy qz qw ..)
+    float pxs[8], pys[8], xrs[8], yus[8], deps[8];
+    if (raster_project(c, p0.x, p0.y, p0.z, p0.w, p1.x, p1.y, p1.z, pxs, pys, xrs, yus, deps)) {
+      RasterEdges E;
+      raster_edges(pxs, pys, E);
+      raster_row_span(E, band * 32 + lane, ln, rn);
+    } else {
+      clipped_row_span(c, pxs, pys, xrs, yus, deps, s_pts[threadIdx.x >> 5], band * 32 + lane, ln, rn);
+    }
+    ln = max(ln, 0); rn = min(rn, res - 1);  // (the float -> int conversions saturate far outside the image)
+  }
+  const int rows = min(32, res - band * 32);
+  const int chunks = rows * res * C / 16;  // whole: res % 4 == 0
+  uint4* out = reinterpret_cast<uint4*>(a.frames + ((f * res + band * 32) * res) * C);
+  for (int c0 = 0; c0 < chunks; c0 += 32) {
+    const int ch = c0 + lane, p = ch * PPC, r = p / res, col = p - r * res;  // first pixel of the chunk: row r (of the band), column col
+    // a mask chunk runs into the next row when res % 16 != 0
+    const int l0 = __shfl_sync(0xFFFFFFFFu, ln, r & 31), r0 = __shfl_sync(0xFFFFFFFFu, rn, r & 31);
+    const int l1 = __shfl_sync(0xFFFFFFFFu, ln, (r + 1) & 31), r1 = __shfl_sync(0xFFFFFFFFu, rn, (r + 1) & 31);
+    if (ch >= chunks) continue;
+    const int wrap = res - col;  // pixels of the chunk still in row r
+    uint32_t bits = run_bits(max(l0 - col, 0), min(min(r0 - col, wrap - 1), PPC - 1));
+    if (wrap < PPC) bits |= run_bits(max(l1 + wrap, wrap), min(r1 + wrap, PPC - 1));
+    uint4 v;
+    if (FMT == QX_FRAME_RGBA) {
+      v.x = bits & 1u ? kRgbaBox : kRgbaSky; v.y = bits & 2u ? kRgbaBox : kRgbaSky;
+      v.z = bits & 4u ? kRgbaBox : kRgbaSky; v.w = bits & 8u ? kRgbaBox : kRgbaSky;
+    } else {  // 4 bits -> 4 bytes of 0 / 255
+      v.x = ((bits & 0xFu) * 0x00204081u & 0x01010101u) * 255u;
+      v.y = ((bits >> 4 & 0xFu) * 0x00204081u & 0x01010101u) * 255u;
+      v.z = ((bits >> 8 & 0xFu) * 0x00204081u & 0x01010101u) * 255u;
+      v.w = ((bits >> 12 & 0xFu) * 0x00204081u & 0x01010101u) * 255u;
+    }
+    __stcs(out + ch, v);
+  }
+}
+
 }  // namespace qx
 
 // ===========================================================================
@@ -1401,6 +1515,29 @@ extern "C" int qx_step(QxHandle* h, const float* actions_dev, void* obs_dev, int
 extern "C" int qx_debug_clock_probe(unsigned long long* out_dev, void* stream) {
   if (!out_dev) return fail(QX_EINVAL, "qx_debug_clock_probe: null buffer");
   qx::clock_probe_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(out_dev);
+  QX_CUDA(cudaGetLastError());
+  return QX_OK;
+}
+
+extern "C" int qx_render(QxHandle* h, const int32_t* env_idx_dev, int64_t m, int32_t fmt, uint8_t* frames_dev, void* stream) {
+  if (!h) return fail(QX_EINVAL, "qx_render: null handle");
+  if (h->dev.task != QX_TASK_HOVER) return fail(QX_EINVAL, "qx_render: camera frames are drawn for the hover task only");
+  if (fmt != QX_FRAME_RGBA && fmt != QX_FRAME_MASK) return fail(QX_EINVAL, "qx_render: fmt is QX_FRAME_RGBA or QX_FRAME_MASK");
+  if (m < 0) return fail(QX_EINVAL, "qx_render: m < 0");
+  if (!env_idx_dev && m != h->n) return fail(QX_EINVAL, "qx_render: env_idx_dev is NULL, so m must equal n_envs");
+  const int res = (int)h->cfg.cam_res;
+  if (!(h->cfg.cam_res >= 4.f && h->cfg.cam_res <= 8192.f) || (float)res != h->cfg.cam_res || res % 4 != 0)
+    return fail(QX_EINVAL, "qx_render: cam_res must be a positive multiple of 4");
+  if (!frames_dev && m > 0) return fail(QX_EINVAL, "qx_render: null frames_dev");
+  if (reinterpret_cast<uintptr_t>(frames_dev) % 16 != 0) return fail(QX_EINVAL, "qx_render: frames_dev must be 16-byte aligned");
+  if (m == 0) return QX_OK;
+  qx::RenderArgs a{h->state, h->n, env_idx_dev, m, frames_dev, res, h->raster};
+  const int64_t warps = m * ((res + 31) / 32);
+  const unsigned grid = (unsigned)((warps + qx::kRenderBlock / 32 - 1) / (qx::kRenderBlock / 32));
+  // a plain launch: the step kernels release their programmatic dependents before they store the state planes read here
+  if (fmt == QX_FRAME_RGBA) qx::render_kernel<QX_FRAME_RGBA><<<grid, qx::kRenderBlock, 0, (cudaStream_t)stream>>>(a);
+  else qx::render_kernel<QX_FRAME_MASK><<<grid, qx::kRenderBlock, 0, (cudaStream_t)stream>>>(a);
+  ++g_launches;
   QX_CUDA(cudaGetLastError());
   return QX_OK;
 }

@@ -834,9 +834,13 @@ __device__ __forceinline__ void vision(const Env& e, const DevConfig& c, bool& v
 // (its constants live in a small device buffer: passing the DevConfig by reference would force the specialised kernels to
 // materialise their literal-folded copy of it in local memory, and 35 by-value arguments would cost the callers registers)
 struct RasterConsts { float cam_sd, cam_cd, inv_tan, res, half_res, inv_half_res, inv_res2, cam_near, cam_off[3], pad, panel[12], panel_back[12]; };
-static __device__ __noinline__ void vision_raster(const float px_w, const float py_w, const float pz_w, const float x, const float y, const float z,
-                                                  const float w, const float* __restrict__ consts, bool& vis, float& cx, float& cy, float& area, float& ratio) {
-  const RasterConsts c = *reinterpret_cast<const RasterConsts*>(consts);
+
+// The two steps of the silhouette raster that vision_raster and the camera-frame kernel share, so that a drawn frame covers
+// exactly the pixels vision_raster counts.  raster_project: the 8 box corners (front face, then back face) in camera space --
+// xr right, yu up, dep along the view axis -- and in continuous pixel coordinates (row 0 = top); returns whether every corner
+// is in front of the near plane (otherwise pxs / pys of the corners behind it are meaningless).
+QX_DI bool raster_project(const RasterConsts& c, const float px_w, const float py_w, const float pz_w, const float x, const float y,
+                          const float z, const float w, float (&pxs)[8], float (&pys)[8], float (&xrs)[8], float (&yus)[8], float (&deps)[8]) {
   const float* panel_front = c.panel;
   const float* panel_back = c.panel_back;
   const float xx = x * x, yy = y * y, zz = z * z, xy = x * y, xz = x * z, yz = y * z, wx = w * x, wy = w * y, wz = w * z;
@@ -852,7 +856,6 @@ static __device__ __noinline__ void vision_raster(const float px_w, const float 
   const float fx = cd, fy = sd * sph, fzz = sd * cph;
   const float ux = -sd * cph, uy = sph * cph * (cd - 1.f), uz = fmaf(sph, sph, cd * cph * cph);
   const float rx = fy * uz - fzz * uy, ry = fzz * ux - fx * uz, rz = fx * uy - fy * ux;
-  float pxs[8], pys[8];
   bool ok = true;
 #pragma unroll
   for (int k = 0; k < 8; ++k) {
@@ -864,9 +867,48 @@ static __device__ __noinline__ void vision_raster(const float px_w, const float 
     const float depth = fx * bx + fy * by + fzz * bz;
     ok = ok && (depth > c.cam_near);
     const float k1 = c.inv_tan / fmaxf(depth, 1e-9f);
-    pxs[k] = fmaf((rx * bx + ry * by + rz * bz) * k1, c.half_res, c.half_res);
-    pys[k] = fmaf(-(ux * bx + uy * by + uz * bz) * k1, c.half_res, c.half_res);
+    const float xr = rx * bx + ry * by + rz * bz;
+    pxs[k] = fmaf(xr * k1, c.half_res, c.half_res);
+    const float yu = ux * bx + uy * by + uz * bz;
+    pys[k] = fmaf(-yu * k1, c.half_res, c.half_res);
+    xrs[k] = xr; yus[k] = yu; deps[k] = depth;
   }
+  return ok;
+}
+
+// the 12 box edges (front ring, back ring, connectors) of projected corners, set up for raster_row_span
+struct RasterEdges { float ex0[12], ey0[12], ey1[12], esl[12]; };
+QX_DI void raster_edges(const float (&pxs)[8], const float (&pys)[8], RasterEdges& E) {
+  constexpr int ea[12] = {0, 1, 2, 3, 4, 5, 6, 7, 0, 1, 2, 3}, eb[12] = {1, 2, 3, 0, 5, 6, 7, 4, 4, 5, 6, 7};
+#pragma unroll
+  for (int k = 0; k < 12; ++k) {
+    E.ex0[k] = pxs[ea[k]]; E.ey0[k] = pys[ea[k]]; E.ey1[k] = pys[eb[k]];
+    const float dy = E.ey1[k] - E.ey0[k];
+    E.esl[k] = dy != 0.f ? (pxs[eb[k]] - pxs[ea[k]]) / dy : 0.f;
+  }
+}
+
+// covered columns [ln, rn] of pixel row r (empty: ln > rn): the silhouette's x interval on the row's centre line y = r + 0.5 is
+// the min / max over the edges crossing it, and a pixel is covered when its centre x + 0.5 lies in that interval
+QX_DI void raster_row_span(const RasterEdges& E, const int r, int& ln, int& rn) {
+  ln = 1; rn = 0;
+  const float yl = (float)r + 0.5f;
+  float xl = 3.0e38f, xr = -3.0e38f;
+#pragma unroll
+  for (int k = 0; k < 12; ++k) {
+    if ((E.ey0[k] - yl) * (E.ey1[k] - yl) <= 0.f && E.ey0[k] != E.ey1[k]) {
+      const float xi = fmaf(yl - E.ey0[k], E.esl[k], E.ex0[k]);
+      xl = fminf(xl, xi); xr = fmaxf(xr, xi);
+    }
+  }
+  if (xl <= xr) { ln = (int)ceilf(xl - 0.5f); rn = (int)floorf(xr - 0.5f); }
+}
+
+static __device__ __noinline__ void vision_raster(const float px_w, const float py_w, const float pz_w, const float x, const float y, const float z,
+                                                  const float w, const float* __restrict__ consts, bool& vis, float& cx, float& cy, float& area, float& ratio) {
+  const RasterConsts c = *reinterpret_cast<const RasterConsts*>(consts);
+  float pxs[8], pys[8], xrs[8], yus[8], deps[8];
+  const bool ok = raster_project(c, px_w, py_w, pz_w, x, y, z, w, pxs, pys, xrs, yus, deps);
   vis = false; cx = cy = area = ratio = 0.f;
   if (!ok) return;
   float ymin = pys[0], ymax = pys[0];
@@ -875,31 +917,15 @@ static __device__ __noinline__ void vision_raster(const float px_w, const float 
   const int res = (int)c.res;
   int r0 = (int)ceilf(ymin - 0.5f), r1 = (int)floorf(ymax - 0.5f);
   r0 = max(r0, -1); r1 = min(r1, res);  // rows outside the image only matter as "touches the border"
-  // edges: front ring, back ring, connectors
-  constexpr int ea[12] = {0, 1, 2, 3, 4, 5, 6, 7, 0, 1, 2, 3}, eb[12] = {1, 2, 3, 0, 5, 6, 7, 4, 4, 5, 6, 7};
-  float ex0[12], ey0[12], ey1[12], esl[12];
-#pragma unroll
-  for (int k = 0; k < 12; ++k) {
-    ex0[k] = pxs[ea[k]]; ey0[k] = pys[ea[k]]; ey1[k] = pys[eb[k]];
-    const float dy = ey1[k] - ey0[k];
-    esl[k] = dy != 0.f ? (pxs[eb[k]] - pxs[ea[k]]) / dy : 0.f;
-  }
+  RasterEdges E;
+  raster_edges(pxs, pys, E);
   int n_pix = 0, interior = 0, lmin = 1 << 20, rmax = -(1 << 20), first = 1 << 20, last = -(1 << 20);
   int lp = 1, rp = 0, lc = 1, rc = 0;  // spans of the previous and the current row (empty: l > r)
   bool edge = false;
   for (int r = r0; r <= r1 + 1; ++r) {  // one row ahead: the interior count of a row needs its lower neighbour
     int ln = 1, rn = 0;
     if (r <= r1) {
-      const float yl = (float)r + 0.5f;
-      float xl = 3.0e38f, xr = -3.0e38f;
-#pragma unroll
-      for (int k = 0; k < 12; ++k) {
-        if ((ey0[k] - yl) * (ey1[k] - yl) <= 0.f && ey0[k] != ey1[k]) {
-          const float xi = fmaf(yl - ey0[k], esl[k], ex0[k]);
-          xl = fminf(xl, xi); xr = fmaxf(xr, xi);
-        }
-      }
-      if (xl <= xr) { ln = (int)ceilf(xl - 0.5f); rn = (int)floorf(xr - 0.5f); }
+      raster_row_span(E, r, ln, rn);
       if (ln <= rn) {
         n_pix += rn - ln + 1;
         lmin = min(lmin, ln); rmax = max(rmax, rn); first = min(first, r); last = max(last, r);

@@ -21,7 +21,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import QX_OBS_BF16, QX_OBS_F32, QX_STATE_WORDS, QX_STATE_WORDS_CASCADE, QX_TASK_HOVER, QxConfig, check, default_config
+from ._lib import QX_FRAME_MASK, QX_FRAME_RGBA, QX_OBS_BF16, QX_OBS_F32, QX_STATE_WORDS, QX_STATE_WORDS_CASCADE, QX_TASK_HOVER, QxConfig, check, default_config
 
 # names of the 44 carried state words, in plane order (see csrc/qx_model.cuh Env)
 STATE_FIELDS = (
@@ -161,6 +161,30 @@ class QuadXSim:
         self._check(terminated, (k, self.n), torch.uint8, "terminated")
         self._check(truncated, (k, self.n), torch.uint8, "truncated")
         check(self.lib.qx_step_k(self._h, k, _ptr(actions), _ptr(obs), _ptr(reward), _ptr(terminated), _ptr(truncated), self._stream()))
+
+    def render(self, env_idx: torch.Tensor | Sequence[int] | None = None, fmt: str = "rgba", out: torch.Tensor | None = None) -> torch.Tensor:
+        """qx_render: the FPV camera frames of the envs' current poses (those the last observation's camera columns were
+        computed from), u8 on the sim device, on the current stream.  fmt "rgba" -> [m, res, res, 4] (the layout of the
+        reference's rgbaImg), "mask" -> [m, res, res] (255 on the red box: the mask detect_rectangle starts from).
+        env_idx: int32 CUDA tensor or sequence of ints (an index outside [0, n) gives a background frame); None = every env.
+        out: optional caller-owned buffer of that shape."""
+        code = {"rgba": QX_FRAME_RGBA, "mask": QX_FRAME_MASK}.get(fmt)
+        if code is None:
+            raise ValueError(f"fmt must be 'rgba' or 'mask', got {fmt!r}")
+        if env_idx is not None:
+            if isinstance(env_idx, torch.Tensor):
+                self._check(env_idx, (env_idx.numel(),), torch.int32, "env_idx")
+            else:
+                env_idx = torch.tensor(list(env_idx), dtype=torch.int32, device=self.device)
+        m = self.n if env_idx is None else env_idx.numel()
+        res = int(self.cfg.cam_res)
+        shape = (m, res, res, 4) if code == QX_FRAME_RGBA else (m, res, res)
+        if out is None:
+            out = torch.empty(shape, dtype=torch.uint8, device=self.device)
+        else:
+            self._check(out, shape, torch.uint8, "out")
+        check(self.lib.qx_render(self._h, _ptr(env_idx), m, code, _ptr(out), self._stream()))
+        return out
 
     # -- host API ----------------------------------------------------------------
     def reset_host(self, mask: np.ndarray | None = None) -> np.ndarray:
@@ -345,12 +369,19 @@ class QuadXHoverEnv:
     ``honour_flight_mode=True`` is passed: then the drone flies in that PyFlyt
     mode (-1..7, the outer PID loops of cf2x.yaml:21-54; set ``action_scale`` /
     ``thrust_scale`` / ``thrust_bias`` to map the Box(-1, 1) action onto it).
+
+    ``render_mode="rgb_array"`` makes ``render()`` return the FPV camera frame of the current state (``np.uint8``
+    [res, res, 4], what the reference's ``drones[0].rgbaImg`` holds).  It is unrelated to ``render``, which is hover.py's
+    switch of the floor rule (hover.py:283).
     """
 
-    metadata = {"render_modes": []}
+    metadata = {"render_modes": ["rgb_array"]}
 
     def __init__(self, flight_mode: int = 0, agent_hz: int = 40, render: bool = False, seed: int = 0, device=None,
-                 honour_flight_mode: bool = False, **cfg_overrides):
+                 honour_flight_mode: bool = False, render_mode: str | None = None, **cfg_overrides):
+        if render_mode not in (None, "rgb_array"):
+            raise ValueError(f"render_mode must be None or 'rgb_array', got {render_mode!r}")
+        self.render_mode = render_mode
         self.flight_mode = flight_mode
         self.agent_hz = agent_hz
         cfg = default_config(QX_TASK_HOVER)
@@ -380,7 +411,9 @@ class QuadXHoverEnv:
         return self.state, float(rew[0]), bool(te[0]), bool(tr[0]), self.info
 
     def render(self):
-        raise NotImplementedError("rendering is out of scope (SURVEY 2, row 6/11)")
+        if self.render_mode != "rgb_array":
+            raise NotImplementedError("rendering is out of scope (SURVEY 2, row 6/11)")
+        return self.sim.render().cpu().numpy()[0]
 
     def close(self):
         self.sim.close()

@@ -39,6 +39,8 @@ extern "C" {
 enum { QX_OK = 0, QX_EINVAL = -1, QX_ECUDA = -2, QX_ENOMEM = -3, QX_EARCH = -4 };
 enum { QX_TASK_HOVER = 0, QX_TASK_YAW = 1 };
 enum { QX_OBS_F32 = 0, QX_OBS_BF16 = 1 };
+#define QX_FRAME_RGBA 0
+#define QX_FRAME_MASK 1
 
 /* Parameters of one simulation.  Defaults (qx_default_config) are the literals
  * of hover.py:23-51,77-110, cf2x.yaml:1-19 and cf2x.urdf:10-68; every field the
@@ -116,7 +118,8 @@ typedef struct QxConfig {
   /* --- camera features (hover.py:157-222).  0: analytic projection of the four front-face corners with pixel-lattice
    * corrections (default, cheapest).  1: scan conversion of the box silhouette on the 128 x 128 lattice and the contour
    * features as cv2 reports them for the rendered frame -- visibility, contour area and bounding-box ratio equal the
-   * reference's detect_rectangle on rasterised frames; ~1.5x the step cost. ------------------------------------------- */
+   * reference's detect_rectangle on rasterised frames; ~1.5x the step cost.  qx_render draws the frame in either mode (its
+   * pixels are the ones mode 1 counts). ----------------------------------------------------------------------------------- */
   int32_t vision_mode;
   float panel_back[12];       /* the 4 corners of the box face behind panel[] (hover.py:118-147: 0.04 deep) */
 } QxConfig;
@@ -160,6 +163,15 @@ int qx_step_begin(QxHandle* h, const float* actions_dev, void* obs_dev, int32_t 
                   float* reward_dev, uint8_t* terminated_dev, uint8_t* truncated_dev, float* terminal_obs_dev, void* stream);
 int qx_step_end(QxHandle* h, void* obs_dev, int32_t obs_dtype, int64_t obs_stride, void* stream);
 int qx_done_queue(QxHandle* h, const uint32_t** count_dev, const uint32_t** idx_dev);
+
+/* The FPV camera frame (Camera.capture_image -> drones[0].rgbaImg, read by detect_rectangle hover.py:157-222) of m envs,
+ * drawn from their current pose: frames_dev u8 [m, res, res, 4] (RGBA) or [m, res, res] (MASK), res = cfg.cam_res.
+ * env_idx_dev: int32 [m] device indices, or NULL for all envs (m must then equal n_envs); an index outside [0, n_envs)
+ * gets a background frame.  Hover task only.  Enqueued on `stream`, no synchronisation, graph-capturable.
+ * frames_dev must be 16-byte aligned (the frames are written with 16-byte stores).  Row 0 is the top of the image.
+ * RGBA: box (200, 0, 0, 255) on (170, 190, 230, 255); MASK: 255 on the box, 0 elsewhere (hover.py:173-177's red mask).  A pixel is on the box when its centre is inside the box's silhouette -- the pixels
+ * vision_mode = 1 counts; a box crossing the camera's near plane is clipped to it. */
+int qx_render(QxHandle* h, const int32_t* env_idx_dev, int64_t m, int32_t fmt, uint8_t* frames_dev, void* stream);
 
 /* k consecutive qx_step in one launch with the state kept in registers
  * (physics-only benchmarking, SURVEY 8d): actions_dev f32 [k, n, act_dim],
