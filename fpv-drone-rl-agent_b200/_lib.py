@@ -98,6 +98,7 @@ def lib() -> C.CDLL:
         "qx_set_state": (C.c_int, [vp, vp]),
         "qx_get_flags": (C.c_int, [vp, i64, i64, vp]),
         "qx_episode_stats": (C.c_int, [vp, C.POINTER(C.c_double), C.POINTER(i64), C.POINTER(i64), i32]),
+        "qx_episode_record": (C.c_int, [vp, f32p, vp, vp, vp, vp]),
         "qx_nonfinite_count": (C.c_int, [vp, C.POINTER(i64)]),
         "qx_num_envs": (i64, [vp]),
         "qx_obs_dim": (i32, [vp]),
@@ -145,7 +146,7 @@ def lib() -> C.CDLL:
 
 EXPORTED = [
     "qx_default_config", "qx_create", "qx_destroy", "qx_reset", "qx_step", "qx_step_begin", "qx_step_end", "qx_done_queue", "qx_step_k", "qx_render", "qx_reset_host", "qx_step_host", "qx_step_host_ex",
-    "qx_get_state", "qx_set_state", "qx_get_flags", "qx_episode_stats", "qx_nonfinite_count", "qx_num_envs", "qx_obs_dim", "qx_act_dim", "qx_state_ptr", "qx_state_words", "qx_uses_reference_constants", "qx_config_matches_reference_constants",
+    "qx_get_state", "qx_set_state", "qx_get_flags", "qx_episode_stats", "qx_episode_record", "qx_nonfinite_count", "qx_num_envs", "qx_obs_dim", "qx_act_dim", "qx_state_ptr", "qx_state_words", "qx_uses_reference_constants", "qx_config_matches_reference_constants",
     "qx_launch_count", "qx_sizeof_config", "qx_last_error", "qx_version",
 ]
 PPO_EXPORTED = ["ppo_policy_forward", "ppo_policy_forward_stats", "ppo_bootstrap_truncated", "ppo_bootstrap_truncated_first", "ppo_reward_normalize_add", "ppo_gae", "ppo_running_stats_update", "ppo_running_stats_scratch_bytes",

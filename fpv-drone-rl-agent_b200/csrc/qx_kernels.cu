@@ -992,6 +992,29 @@ __global__ void __launch_bounds__(kRenderBlock) render_kernel(const __grid_const
   }
 }
 
+// ---------------------------------------------------------------------------
+// K7: the evaluation ledger (qx_episode_record).  One thread per env, after every step of a handle without auto-reset: an
+// open record whose env's flags word says the episode ended is closed with the return and length the state holds at that
+// step -- later steps of the frozen env keep adding to ep_ret and step_count, so the result exists only on this step.  An
+// open record costs one 16-byte load (plane 7), a closing one a second (plane 8), a closed one only its own end word.
+// ---------------------------------------------------------------------------
+constexpr int kRecordBlock = 256;
+__global__ void __launch_bounds__(kRecordBlock) episode_record_kernel(const float4* __restrict__ state, const int64_t n, float* __restrict__ ret,
+                                                                      int32_t* __restrict__ len, uint32_t* __restrict__ end,
+                                                                      uint32_t* __restrict__ n_closed) {
+  const int64_t i = (int64_t)blockIdx.x * kRecordBlock + threadIdx.x;
+  if (i >= n || end[i] != 0u) return;
+  const float4 p7 = state[7 * n + i];  // (svb2, step_count, rng_ctr, flags)
+  const uint32_t fl = __float_as_uint(p7.w);
+  if (!(fl & (F_TERM | F_TRUNC))) return;
+  ret[i] = state[8 * n + i].w;  // (peul0, peul1, peul2, ep_ret)
+  len[i] = __float_as_int(p7.y);
+  end[i] = fl;
+  // envs that end together (a mass floor termination) count with one atomic per warp, as episode_end does
+  const auto g = cooperative_groups::coalesced_threads();
+  if (g.thread_rank() == 0) atomicAdd(n_closed, g.size());
+}
+
 }  // namespace qx
 
 // ===========================================================================
@@ -1537,6 +1560,19 @@ extern "C" int qx_render(QxHandle* h, const int32_t* env_idx_dev, int64_t m, int
   // a plain launch: the step kernels release their programmatic dependents before they store the state planes read here
   if (fmt == QX_FRAME_RGBA) qx::render_kernel<QX_FRAME_RGBA><<<grid, qx::kRenderBlock, 0, (cudaStream_t)stream>>>(a);
   else qx::render_kernel<QX_FRAME_MASK><<<grid, qx::kRenderBlock, 0, (cudaStream_t)stream>>>(a);
+  ++g_launches;
+  QX_CUDA(cudaGetLastError());
+  return QX_OK;
+}
+
+extern "C" int qx_episode_record(QxHandle* h, float* ret_dev, int32_t* len_dev, uint32_t* end_dev, uint32_t* n_closed_dev, void* stream) {
+  if (!h) return fail(QX_EINVAL, "qx_episode_record: null handle");
+  // with auto-reset the reset of a finished env clears its flags word (and its return) before a record could see them
+  if (h->cfg.auto_reset) return fail(QX_EINVAL, "qx_episode_record: the handle must be created with auto_reset = 0");
+  if (!ret_dev || !len_dev || !end_dev || !n_closed_dev) return fail(QX_EINVAL, "qx_episode_record: null output pointer");
+  const unsigned grid = (unsigned)((h->n + qx::kRecordBlock - 1) / qx::kRecordBlock);
+  // a plain launch: it starts after the step launch before it has stored the state planes
+  qx::episode_record_kernel<<<grid, qx::kRecordBlock, 0, (cudaStream_t)stream>>>(h->state, h->n, ret_dev, len_dev, end_dev, n_closed_dev);
   ++g_launches;
   QX_CUDA(cudaGetLastError());
   return QX_OK;

@@ -186,6 +186,17 @@ class QuadXSim:
         check(self.lib.qx_render(self._h, _ptr(env_idx), m, code, _ptr(out), self._stream()))
         return out
 
+    def episode_record(self, ret: torch.Tensor, length: torch.Tensor, end: torch.Tensor, n_closed: torch.Tensor) -> None:
+        """qx_episode_record on the current stream (a sim with auto_reset = 0, after every step): the open records (end == 0)
+        of envs whose episode has ended are closed with the episode's return (f32 [n]), length (int32 [n]) and flags word
+        (int32 [n], the bits of qx_get_flags, never 0 once closed); n_closed (int32 [1]) counts the closed records.  Zero
+        `end` and `n_closed` before the first step of an evaluation."""
+        self._check(ret, (self.n,), torch.float32, "ret")
+        self._check(length, (self.n,), torch.int32, "length")
+        self._check(end, (self.n,), torch.int32, "end")  # u32 words on the device; the flag bits stay below bit 31
+        self._check(n_closed, (1,), torch.int32, "n_closed")
+        check(self.lib.qx_episode_record(self._h, _ptr(ret), _ptr(length), _ptr(end), _ptr(n_closed), self._stream()))
+
     # -- host API ----------------------------------------------------------------
     def reset_host(self, mask: np.ndarray | None = None) -> np.ndarray:
         obs = np.empty((self.n, self.obs_dim), np.float32)

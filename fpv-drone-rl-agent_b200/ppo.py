@@ -278,6 +278,128 @@ def policy_forward(pol: PackedPolicy, obs: torch.Tensor, *, obs_stats: RunningSt
                                         _stream(pol.device)))
 
 
+F_TERMINATED, F_TRUNCATED, F_OUT_OF_BOUNDS, F_ON_FLOOR = 2, 4, 8, 16  # bits of the flags word (qx_get_flags)
+
+
+class PolicyEvaluator:
+    """SB3 ``evaluate_policy(model, env, n_eval_episodes, deterministic=True)`` -- the playback loop of test_hover.py:13-27 --
+    on the device.  The evaluator owns a sim of ``n_episodes`` envs (auto_reset = 0, env ids 0 .. n_episodes - 1, the caller's
+    env config otherwise) and every env flies exactly one episode, so short episodes are not over-represented as they are when
+    finished episodes are counted until n_eval_episodes is reached.  Each step is the deterministic policy (a = mean, clipped to
+    the action box) on observations normalised with a frozen copy of ``obs_stats`` (VecNormalize with training=False; rewards
+    are the raw env rewards, norm_reward=False), the env step, and qx_episode_record, which latches each episode's return,
+    length and end flags on the step it ends.
+
+    A chunk of ``chunk`` such steps is one CUDA-graph replay (``use_cuda_graph=False``: eager launches, same results); the host
+    reads the number of closed records once per chunk.  Every ``evaluate()`` starts from the state the first reset produced,
+    motor-noise counters included, so two evaluations of the same policy give the same numbers.  The packed policy is read
+    where it lives: an evaluator built once follows the weights of a policy that keeps training."""
+
+    def __init__(self, policy: PackedPolicy, obs_stats: RunningStats | None, env_cfg=None, n_episodes: int = 4096, seed: int = 0,
+                 task: int = 0, obs_clip: float = 10.0, device=None, chunk: int = 32, use_cuda_graph: bool = True):
+        from ._lib import QxConfig, default_config
+
+        if n_episodes <= 0 or chunk <= 0:
+            raise ValueError("n_episodes and chunk must be positive")
+        cfg = default_config(task) if env_cfg is None else QxConfig.from_buffer_copy(env_cfg)
+        if cfg.task != task:
+            raise ValueError(f"env_cfg is for task {cfg.task}, the evaluator was asked for task {task}")
+        cfg.update(auto_reset=0)
+        self.sim = QuadXSim(n_episodes, cfg, seed=seed, env_id0=0, device=policy.device if device is None else device)
+        if (policy.struct.obs_dim, policy.struct.act_dim) != (self.sim.obs_dim, self.sim.act_dim):
+            self.sim.close()
+            raise ValueError(f"policy has obs_dim {policy.struct.obs_dim}, act_dim {policy.struct.act_dim}; task {task} needs "
+                             f"{self.sim.obs_dim}, {self.sim.act_dim}")
+        if obs_stats is not None and obs_stats.dim != self.sim.obs_dim:
+            self.sim.close()
+            raise ValueError(f"obs_stats has dim {obs_stats.dim}, task {task} observations have {self.sim.obs_dim}")
+        self.pol, self.obs_stats, self.obs_clip = policy, obs_stats, float(obs_clip)
+        self.n, self.seed, self.chunk, self.use_cuda_graph = int(n_episodes), int(seed), int(chunk), bool(use_cuda_graph)
+        n, d = self.n, self.sim.device
+        self.device = d
+        self.obs = torch.zeros(n, self.sim.obs_dim, device=d)
+        self.env_actions = torch.zeros(n, self.sim.act_dim, device=d)
+        self.reward = torch.zeros(n, device=d)
+        self.te = torch.zeros(n, dtype=torch.uint8, device=d)
+        self.tr = torch.zeros(n, dtype=torch.uint8, device=d)
+        self.ret = torch.zeros(n, device=d)
+        self.length = torch.zeros(n, dtype=torch.int32, device=d)
+        self.end = torch.zeros(n, dtype=torch.int32, device=d)
+        self.n_closed = torch.zeros(1, dtype=torch.int32, device=d)
+        self.norm = (torch.zeros(self.sim.obs_dim, device=d), torch.ones(self.sim.obs_dim, device=d)) if obs_stats is not None else None
+        self.sim.reset(self.obs)
+        self._obs0 = self.obs.clone()
+        self._state0 = self.sim.get_state()
+        self._graph = None
+        # one-time kernel attribute setup must not happen inside a graph capture
+        policy_forward(self.pol, self.obs, norm=self.norm, obs_clip=self.obs_clip, deterministic=True, env_actions=self.env_actions)
+
+    def _chunk(self) -> None:
+        for _ in range(self.chunk):
+            policy_forward(self.pol, self.obs, norm=self.norm, obs_clip=self.obs_clip, deterministic=True, env_actions=self.env_actions)
+            self.sim.step(self.env_actions, self.obs, self.reward, self.te, self.tr)
+            self.sim.episode_record(self.ret, self.length, self.end, self.n_closed)
+
+    def _run_chunk(self) -> None:
+        if not self.use_cuda_graph:
+            self._chunk()
+            return
+        if self._graph is None:
+            st = torch.cuda.Stream(device=self.device)
+            st.wait_stream(torch.cuda.current_stream(self.device))
+            with torch.cuda.stream(st):
+                g = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(g, stream=st):
+                    self._chunk()
+            torch.cuda.current_stream(self.device).wait_stream(st)
+            self._graph = g
+        self._graph.replay()
+
+    def evaluate(self) -> tuple[dict, dict]:
+        """Fly every env's episode from the initial state.  Returns (summary, records): summary holds evaluate_policy's
+        mean_reward / std_reward (population std, as np.std), mean_ep_length, success_rate (truncated by the time limit and not
+        terminated), floor_rate (floor rule), oob_rate (left the flight dome), n_episodes and the steps run; records holds
+        the per-episode tensors return (f32), length (int32) and end (int32 flags word), one entry per env."""
+        self.sim.set_state(self._state0)
+        self.obs.copy_(self._obs0)
+        if self.norm is not None:
+            self.norm[0].copy_(self.obs_stats.mean)
+            self.norm[1].copy_(self.obs_stats.inv_std)
+        for t in (self.ret, self.length, self.end, self.n_closed):
+            t.zero_()
+        limit, steps = int(self.sim.cfg.max_steps) + 2, 0  # the hover time limit ends an episode on step max_steps + 2
+        while True:
+            self._run_chunk()
+            steps += self.chunk
+            closed = int(self.n_closed.item())
+            if closed == self.n:
+                break
+            if steps >= limit:
+                raise RuntimeError(f"{self.n - closed} of {self.n} episodes still open after {steps} steps (every episode ends by step {limit})")
+        ret = self.ret.double().cpu()
+        end = self.end.cpu()
+        trunc, term = (end & F_TRUNCATED) != 0, (end & F_TERMINATED) != 0
+        summary = {"mean_reward": float(ret.mean()), "std_reward": float(ret.std(correction=0)),
+                   "mean_ep_length": float(self.length.double().mean()), "success_rate": float((trunc & ~term).double().mean()),
+                   "floor_rate": float(((end & F_ON_FLOOR) != 0).double().mean()), "oob_rate": float(((end & F_OUT_OF_BOUNDS) != 0).double().mean()),
+                   "n_episodes": self.n, "steps": steps}
+        return summary, {"return": self.ret.clone(), "length": self.length.clone(), "end": self.end.clone()}
+
+    def close(self) -> None:
+        self._graph = None
+        self.sim.close()
+
+
+def evaluate_policy(policy: PackedPolicy, obs_stats: RunningStats | None, env_cfg=None, n_episodes: int = 4096, seed: int = 0,
+                    task: int = 0, obs_clip: float = 10.0, device=None, **kw) -> tuple[dict, dict]:
+    """One evaluation with a PolicyEvaluator built for it (kw: chunk, use_cuda_graph); (summary, records) as evaluate()."""
+    ev = PolicyEvaluator(policy, obs_stats, env_cfg, n_episodes, seed, task, obs_clip, device, **kw)
+    try:
+        return ev.evaluate()
+    finally:
+        ev.close()
+
+
 def gae(rewards, values, dones, last_values, gamma: float, lam: float, advantages, returns) -> None:
     """``RolloutBuffer.compute_returns_and_advantage`` (ppo_gae); all [T, n] contiguous."""
     T, n = rewards.shape
@@ -608,6 +730,7 @@ class PPOTrainer:
         self.num_timesteps = 0
         self._iteration = 0
         self._flat_grad = None
+        self._evaluator = None  # PolicyEvaluator of evaluate(), built on its first call
         self.gen = torch.Generator(device=dev).manual_seed(cfg.seed + 1000 + rank)
 
     def _allreduce_grads(self) -> None:
@@ -800,6 +923,21 @@ class PPOTrainer:
         out.update(ep_rew_mean=s / c if c else float("nan"), ep_len_mean=l / c if c else float("nan"), episodes=int(c),
                    timesteps=self.num_timesteps)
         return out
+
+    def evaluate(self, n_episodes: int = 4096, seed: int | None = None) -> tuple[dict, dict]:
+        """EvalCallback's evaluation of the current policy: PolicyEvaluator on the trainer's packed weights, its VecNormalize
+        observation statistics (frozen for the evaluation), clip_obs, task and env config; seed None = cfg.seed + 1.  The
+        evaluator (its own sim and graph) is built on the first call and kept while (n_episodes, seed) stay the same.  Reads the
+        policy and the statistics only: no rollout buffer, statistic, random stream or env of training changes."""
+        seed = self.cfg.seed + 1 if seed is None else int(seed)
+        ev = self._evaluator
+        if ev is None or (ev.n, ev.seed) != (n_episodes, seed):
+            if ev is not None:
+                ev.close()
+            ev = PolicyEvaluator(self.packed, self.rollout.obs_stats if self.cfg.norm_obs else None, self.sim.cfg, n_episodes, seed,
+                                 task=self.sim.cfg.task, obs_clip=self.cfg.clip_obs, device=self.device)
+            self._evaluator = ev
+        return ev.evaluate()
 
     def save(self, path: str) -> None:
         """Counterpart of model.save + env.save (train_hover.py:26-27,62-63): policy, optimiser, VecNormalize statistics, and

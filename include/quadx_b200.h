@@ -205,6 +205,16 @@ int32_t qx_state_words(const QxHandle* h);
  * sums over the episodes finished since the last call with clear != 0. */
 int qx_episode_stats(QxHandle* h, double* sum_return, int64_t* sum_length, int64_t* n_episodes, int32_t clear);
 
+/* Evaluation ledger (SB3 evaluate_policy / Monitor per episode; test_hover.py:13-27): for a handle created with
+ * cfg.auto_reset == 0, call after every qx_step.  Env i whose record is open (end_dev[i] == 0) and whose episode has
+ * ended (flags word: terminated | truncated) closes it: ret_dev[i] = its episode return (the ep_ret word), len_dev[i] =
+ * step_count, end_dev[i] = the flags word (bits as qx_get_flags; never 0 once closed), and *n_closed_dev += 1.
+ * Closed records are never written again.  The caller zero-fills end_dev and *n_closed_dev before the first step.
+ * ret_dev f32 [n_envs], len_dev i32 [n_envs], end_dev u32 [n_envs], n_closed_dev u32 [1].  Any task, flight or vision
+ * mode.  Enqueued on `stream`, no allocation, no synchronisation, graph-capturable; QX_EINVAL (nothing launched) for a
+ * null handle, a handle with auto_reset != 0 or a null output. */
+int qx_episode_record(QxHandle* h, float* ret_dev, int32_t* len_dev, uint32_t* end_dev, uint32_t* n_closed_dev, void* stream);
+
 /* Failure detection (no reference counterpart): envs whose state stopped being finite since creation; each was
  * terminated like an out-of-bounds flight and re-created by the auto-reset. */
 int qx_nonfinite_count(QxHandle* h, int64_t* count);

@@ -11,6 +11,8 @@ What the reference script does -> here:
   CheckpointCallback(min 20 000 steps, name with loss/len/rew) -> same cadence and file naming, torch .pt files
   tensorboard_log="./tensorboard"                 -> same tags (rollout/ep_len_mean, rollout/ep_rew_mean, time/fps, train/*)
   model.save("hover"); env.save("hover")          -> hover.pt (policy + optimiser + normalisation statistics)
+  EvalCallback (SB3; not in the reference script) -> --eval-every K: deterministic evaluation on the device (ppo.PolicyEvaluator),
+                                                     eval/mean_reward, eval/mean_ep_length, eval/success_rate
 """
 from __future__ import annotations
 
@@ -51,7 +53,12 @@ def main():
     ap.add_argument("--log-std-min-final", type=float, default=None, help="... released linearly to this value ...")
     ap.add_argument("--log-std-min-iters", type=int, nargs=2, default=(0, 0), help="... between these iterations")
     ap.add_argument("--json", default="", help="write the per-iteration log here")
+    ap.add_argument("--eval-every", type=int, default=0, help="evaluate the deterministic policy every K iterations and after training "
+                                                                 "(EvalCallback; rank 0 only; 0 = off)")
+    ap.add_argument("--eval-episodes", type=int, default=4096, help="episodes per evaluation (one env each)")
+    ap.add_argument("--eval-seed", type=int, default=None, help="seed of the evaluation envs (default: --seed + 1)")
     args = ap.parse_args()
+    eval_seed = args.seed + 1 if args.eval_seed is None else args.eval_seed
 
     import torch
     import torch.distributed as dist
@@ -80,11 +87,25 @@ def main():
         writer = SummaryWriter(args.tensorboard)
     if rank == 0:
         os.makedirs(args.save_path, exist_ok=True)
-    last_ckpt, log, t0 = 0, [], time.time()
+    last_ckpt, log, t0, eval_s = 0, [], time.time(), 0.0
+
+    def evaluate(out):
+        """EvalCallback: the deterministic policy on its own envs; the summary goes into this iteration's log entry"""
+        nonlocal eval_s
+        te = time.time()
+        ev, _ = trainer.evaluate(args.eval_episodes, eval_seed)
+        eval_s += time.time() - te  # kept out of wall_s / fps, which stay the training rate
+        out["eval"] = ev
+        print(f"eval {out['timesteps']:>12,d} steps: mean_reward {ev['mean_reward']:9.2f} +/- {ev['std_reward']:.2f} mean_ep_length {ev['mean_ep_length']:7.1f} "
+              f"success {ev['success_rate']:.3f} floor {ev['floor_rate']:.3f} oob {ev['oob_rate']:.3f} ({ev['n_episodes']} episodes)", flush=True)
+        if writer:
+            for tag, key in (("eval/mean_reward", "mean_reward"), ("eval/mean_ep_length", "mean_ep_length"), ("eval/success_rate", "success_rate")):
+                writer.add_scalar(tag, ev[key], out["timesteps"])
+
     for it in range(args.iters):
         out = trainer.learn_iteration()
         torch.cuda.synchronize()
-        out["wall_s"] = time.time() - t0
+        out["wall_s"] = time.time() - t0 - eval_s
         out["fps"] = out["timesteps"] / out["wall_s"]
         if rank == 0:
             if it % args.print_every == 0:
@@ -95,6 +116,8 @@ def main():
                 for tag, key in (("rollout/ep_len_mean", "ep_len_mean"), ("rollout/ep_rew_mean", "ep_rew_mean"), ("time/fps", "fps"),
                                  ("train/policy_gradient_loss", "pg"), ("train/value_loss", "vf"), ("train/approx_kl", "kl"), ("train/clip_fraction", "clipfrac")):
                     writer.add_scalar(tag, out[key], out["timesteps"])
+            if args.eval_every and (it + 1) % args.eval_every == 0:
+                evaluate(out)
             if out["timesteps"] - last_ckpt >= args.min_steps_between_checkpoints:  # train_hover.py:17-31
                 name = f"ppo_hover_{out['timesteps']}_steps_{round(out['vf'], 2)}_len{round(out['ep_len_mean'], 2)}_rew{round(out['ep_rew_mean'], 2)}.pt"
                 trainer.save(os.path.join(args.save_path, name))
@@ -104,6 +127,8 @@ def main():
         if args.total_timesteps and out["timesteps"] >= args.total_timesteps:
             break
     if rank == 0:
+        if args.eval_every and log and "eval" not in log[-1]:  # the trained policy (an evaluation of the same weights would repeat itself)
+            evaluate(log[-1])
         trainer.save("hover.pt")  # train_hover.py:62-63
         trainer.save_sb3("hover_sb3.zip")  # policy.pth under SB3's parameter names + VecNormalize statistics (ppo.export_sb3_zip)
         if args.json:
