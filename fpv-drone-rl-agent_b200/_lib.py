@@ -123,6 +123,7 @@ def lib() -> C.CDLL:
         "ppo_reward_normalize_add": (C.c_int, [vp, vp, vp, vp, i64, f32, f32, f32, vp, vp, vp, vp, vp]),
         "ppo_test_gemm": (C.c_int, [vp, vp, vp, i32, i32, vp]),
         "ppo_test_gemm_mn": (C.c_int, [vp, vp, vp, i32, i32, i32, i32, vp]),
+        "ppo_test_tanh_bf16": (C.c_int, [vp, vp, i64, vp]),
         "ppo_update_num_params": (i32, [i32, i32]),
         "ppo_update_workspace_bytes": (i64, [i32, i32]),
         "ppo_update_minibatch": (C.c_int, [C.POINTER(PpoPolicy), vp, vp, vp, vp, vp, vp, i32, i64, f32, f32, f32, i32, vp, vp, vp, vp]),
@@ -150,7 +151,7 @@ EXPORTED = [
     "qx_launch_count", "qx_sizeof_config", "qx_last_error", "qx_version",
 ]
 PPO_EXPORTED = ["ppo_policy_forward", "ppo_policy_forward_stats", "ppo_bootstrap_truncated", "ppo_bootstrap_truncated_first", "ppo_reward_normalize_add", "ppo_gae", "ppo_running_stats_update", "ppo_running_stats_scratch_bytes",
-                "ppo_reward_normalize", "ppo_test_gemm", "ppo_test_gemm_mn", "ppo_update_num_params", "ppo_update_workspace_bytes",
+                "ppo_reward_normalize", "ppo_test_gemm", "ppo_test_gemm_mn", "ppo_test_tanh_bf16", "ppo_update_num_params", "ppo_update_workspace_bytes",
                 "ppo_update_minibatch", "ppo_update_grad_norm", "ppo_update_adam", "ppo_update_step_count", "ppo_update_set_lr_scale", "ppo_update_kl_stop", "ppo_update_set_log_std_floor", "ppo_update_recompute_logp"]
 
 

@@ -132,6 +132,11 @@ struct FwdArgs {
   float* fs_inv_out;              // == obs_inv_std, writable
   int32_t pdl_wait;               // launched as a programmatic dependent of the statistics kernel: wait for it before reading its results
   int32_t boot_store;             // bootstrap: reward[row] = gamma V (the reward-normalisation launch that follows adds its result) instead of +=
+  // 16-byte vector paths, decided on the host (fwd_vector_flags) so that the branches are uniform: a column slice of a wider
+  // buffer, or a tensor at an odd storage offset, has a base pointer that is not 16-byte aligned and takes the scalar paths
+  int32_t obs_vec;                // obs rows as float4: obs 16-byte aligned and obs_stride % 4 == 0
+  int32_t norm_vec;               // obs_norm_out rows as float4: obs_norm_out 16-byte aligned and obs_dim % 4 == 0
+  int32_t act_vec;                // actions / env_actions rows as float4: act_dim == 4 and both (where given) 16-byte aligned
 };
 
 // (defined with the K4 kernels below)
@@ -154,6 +159,15 @@ __device__ __forceinline__ uint32_t tanh_pack_bf16x2(float lo, float hi) {
   __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
   return *reinterpret_cast<uint32_t*>(&v);
 #endif
+}
+
+// test hook: the hidden epilogue's activation on its own -- out[2i], out[2i + 1] = tanh_pack_bf16x2(x[2i], x[2i + 1]) (lo, hi)
+__global__ void __launch_bounds__(256) test_tanh_kernel(const float* __restrict__ x, uint16_t* __restrict__ out, int64_t n) {
+  const int64_t i = 2 * ((int64_t)blockIdx.x * blockDim.x + threadIdx.x);
+  if (i >= n) return;
+  const uint32_t r = tanh_pack_bf16x2(x[i], i + 1 < n ? x[i + 1] : 0.f);
+  out[i] = (uint16_t)(r & 0xffffu);
+  if (i + 1 < n) out[i + 1] = (uint16_t)(r >> 16);
 }
 
 // optional phase-timing buffer (debug / tuning only, see tools/k2_phases.py): [tile iteration][16] clock64 stamps of CTA 0, slot 0
@@ -191,7 +205,7 @@ __device__ __forceinline__ void load_obs_chunks(const FwdArgs& a, int64_t tile, 
   const int64_t xr = a.gather_idx ? (int64_t)a.gather_idx[tile * 128 + xrow] : tile * 128 + xrow;
   const float* src = a.obs + xr * a.obs_stride + 16 * xh;
   const int c0 = 16 * (int)xh;
-  if ((a.obs_stride & 3) == 0) {
+  if (a.obs_vec) {
 #pragma unroll
     for (int v = 0; v < 4; ++v)
       if (c0 + 4 * v + 4 <= obs_dim) {
@@ -357,7 +371,7 @@ __global__ void __launch_bounds__(kFwdThreads, 1) policy_forward_kernel(const Fw
       *reinterpret_cast<uint4*>(slotp + kSlotX + chunk_off(xrow, q, 128)) = make_uint4(w[0], w[1], w[2], w[3]);
       if (a.obs_norm_out && xvalid) {
         float* dst = a.obs_norm_out + xr * obs_dim + c0;
-        if ((obs_dim & 3) == 0 && c0 + 8 <= obs_dim) {
+        if (a.norm_vec && c0 + 8 <= obs_dim) {
           *reinterpret_cast<float4*>(dst) = make_float4(x[0], x[1], x[2], x[3]);
           *reinterpret_cast<float4*>(dst + 4) = make_float4(x[4], x[5], x[6], x[7]);
         } else {
@@ -403,7 +417,7 @@ __global__ void __launch_bounds__(kFwdThreads, 1) policy_forward_kernel(const Fw
         act[j] = fmaf(__expf(ls), nz[j], mean[j]);
         logp += -0.5f * nz[j] * nz[j] - ls - 0.91893853320467f;
       }
-    if (act_dim == 4) {
+    if (a.act_vec) {
       if (a.actions) *reinterpret_cast<float4*>(a.actions + row * 4) = make_float4(act[0], act[1], act[2], act[3]);
       if (a.env_actions)
         *reinterpret_cast<float4*>(a.env_actions + row * 4) =
@@ -770,7 +784,19 @@ extern "C" int ppo_test_gemm(const void* a, const void* b, float* d, int32_t n, 
   return cudaGetLastError() == cudaSuccess ? QX_OK : pfail(QX_ECUDA, "ppo_test_gemm: launch failed");
 }
 
+extern "C" int ppo_test_tanh_bf16(const float* x, uint16_t* out, int64_t n, void* stream) {
+  if (!x || !out || n <= 0) return pfail(QX_EINVAL, "ppo_test_tanh_bf16: bad arguments");
+  const int64_t pairs = (n + 1) / 2;
+  ppo::test_tanh_kernel<<<(unsigned)((pairs + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, out, n);
+  return cudaGetLastError() == cudaSuccess ? QX_OK : pfail(QX_ECUDA, "ppo_test_tanh_bf16: launch failed");
+}
+
+static bool aligned16(const void* p) { return ((uintptr_t)p & 15u) == 0; }
+
 static int launch_forward(ppo::FwdArgs& a, int64_t max_rows, void* stream) {
+  a.obs_vec = aligned16(a.obs) && (a.obs_stride & 3) == 0;
+  a.norm_vec = (a.p.obs_dim & 3) == 0 && aligned16(a.obs_norm_out);
+  a.act_vec = a.p.act_dim == 4 && aligned16(a.actions) && aligned16(a.env_actions);  // (a null pointer is aligned)
   // per device: SM count and the one-time opt-in to ~200 KB of dynamic shared memory (the attribute is per device; the cached
   // value is set only after the call succeeded, so a failure is retried)
   static std::atomic<int> sms_of[64];

@@ -188,6 +188,7 @@ class PackedPolicy:
         self.b2 = torch.zeros(2 * HID, device=d)
         self.b3 = torch.zeros(HEAD_PAD, device=d)
         self.log_std = torch.zeros(4, device=d)
+        self.device = self.w1.device  # with its index ("cuda" -> "cuda:<current>"): what the outputs of policy_forward must be on
         self.struct = PpoPolicy(self.w1.data_ptr(), self.w2p.data_ptr(), self.w2v.data_ptr(), self.w3.data_ptr(), self.b1.data_ptr(),
                                 self.b2.data_ptr(), self.b3.data_ptr(), self.log_std.data_ptr(), model.obs_dim, model.act_dim)
         self.refresh()
@@ -264,6 +265,13 @@ def policy_forward(pol: PackedPolicy, obs: torch.Tensor, *, obs_stats: RunningSt
     with fused_stats, one launch with the merge inside the policy kernel."""
     n = obs.shape[0]
     assert obs.dtype == torch.float32 and obs.stride(1) == 1
+    # the kernel writes dense [n, act_dim], [n] and [n, obs_dim] arrays from the base pointer: anything else would be written wrongly
+    od, ad, dev = pol.model.obs_dim, pol.model.act_dim, pol.device
+    for name, t, numel in (("actions", actions, n * ad), ("env_actions", env_actions, n * ad), ("values", values, n),
+                           ("log_probs", log_probs, n), ("obs_norm", obs_norm, n * od)):
+        if t is not None and (t.dtype != torch.float32 or t.device != dev or not t.is_contiguous() or t.numel() != numel):
+            raise ValueError(f"policy_forward: {name} must be a contiguous float32 tensor of {numel} elements on {dev}, "
+                             f"got {tuple(t.shape)} {t.dtype} on {t.device} (contiguous: {t.is_contiguous()})")
     mean, inv_std = norm if norm is not None else ((obs_stats.mean, obs_stats.inv_std) if obs_stats else (None, None))
     if update_stats:
         assert obs_stats is not None and mean is not None

@@ -164,6 +164,11 @@ int ppo_test_gemm_mn(const void* a_bf16, const void* b_bf16, float* d, int32_t n
 /* test hook: D[128, n] (fp32) = A[128, k] x B[n, k]^T with one tcgen05.mma chain (bf16 inputs) */
 int ppo_test_gemm(const void* a_bf16, const void* b_bf16, float* d, int32_t n, int32_t k, void* stream);
 
+/* test hook: the policy forward's hidden activation, bf16(tanh(x)) for x[0 .. n), applied pairwise (x[2i] as the low half,
+ * x[2i + 1] as the high half) through the same device function as the kernel's epilogue -- what a reference of the forward
+ * cannot compute itself is the rounding of tanh.approx */
+int ppo_test_tanh_bf16(const float* x, uint16_t* out_bf16, int64_t n, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
