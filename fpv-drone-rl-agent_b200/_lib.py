@@ -8,6 +8,8 @@ from __future__ import annotations
 import ctypes as C
 import os
 
+import torch
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("QX_LIB") or os.path.join(_HERE, "csrc", "libquadx_b200.so")  # QX_LIB: a tuning build (tools/ only)
 
@@ -168,3 +170,30 @@ def default_config(task: int = QX_TASK_HOVER) -> QxConfig:
     cfg = QxConfig()
     check(lib().qx_default_config(task, C.byref(cfg)))
     return cfg
+
+
+def ptr(t: torch.Tensor | None) -> C.c_void_p | None:
+    return None if t is None else C.c_void_p(t.data_ptr())
+
+
+def stream(device: torch.device) -> C.c_void_p:
+    """The current stream of an indexed CUDA device (cuda_device), read as the raw handle (as torch's own generated launchers read
+    it): building a torch.cuda.Stream object first costs a microsecond of host time on every eager launch."""
+    return C.c_void_p(torch._C._cuda_getCurrentRawStream(device.index))
+
+
+def cuda_device(device: int | str | torch.device | None = None) -> torch.device:
+    """None, "cuda", an int or a torch.device -> that CUDA device with its index, as tensors allocated there report it."""
+    dev = torch.device("cuda") if device is None else torch.device(device)
+    if dev.type != "cuda":
+        raise ValueError(f"device must be a CUDA device, got {dev}")
+    return dev if dev.index is not None else torch.device("cuda", torch.cuda.current_device())
+
+
+def expect(t: torch.Tensor, name: str, *, dtype: torch.dtype | tuple, device: torch.device, shape=None, numel: int | None = None) -> None:
+    """Raise ValueError naming `name` unless `t` is a contiguous tensor of `dtype` (or of one in a tuple) on `device`, with `shape`
+    and `numel` where given: the kernels address such buffers densely from the base pointer and would misuse any other."""
+    if ((t.dtype not in dtype if isinstance(dtype, tuple) else t.dtype != dtype) or t.device != device or not t.is_contiguous()
+            or (shape is not None and tuple(t.shape) != tuple(shape)) or (numel is not None and t.numel() != numel)):
+        raise ValueError(f"{name}: expected a contiguous tensor of {dtype}, shape {shape}, {numel} elements on {device}; got "
+                         f"{t.dtype} {tuple(t.shape)} on {t.device} (contiguous: {t.is_contiguous()})")

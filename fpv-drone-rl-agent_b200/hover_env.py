@@ -21,7 +21,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import QX_FRAME_MASK, QX_FRAME_RGBA, QX_OBS_BF16, QX_OBS_F32, QX_STATE_WORDS, QX_STATE_WORDS_CASCADE, QX_TASK_HOVER, QxConfig, check, default_config
+from ._lib import QX_FRAME_MASK, QX_FRAME_RGBA, QX_OBS_BF16, QX_OBS_F32, QX_STATE_WORDS, QX_STATE_WORDS_CASCADE, QX_TASK_HOVER, QxConfig, check, default_config, expect, ptr, stream
 
 # names of the 44 carried state words, in plane order (see csrc/qx_model.cuh Env)
 STATE_FIELDS = (
@@ -62,10 +62,6 @@ class Box:
         return f"Box({self.low.min()}, {self.high.max()}, {self.shape}, {self.dtype})"
 
 
-def _ptr(t: torch.Tensor | None):
-    return None if t is None else C.c_void_p(t.data_ptr())
-
-
 class QuadXSim:
     """Thin owner of one ``QxHandle``: tensors in, tensors out, current torch stream."""
 
@@ -74,10 +70,7 @@ class QuadXSim:
         if not torch.cuda.is_available():
             raise RuntimeError("QuadXSim needs a CUDA device (B200, sm_100a); there is no CPU fallback")
         self.lib = _lib.lib()
-        dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
-        if dev.type != "cuda":
-            raise ValueError("device must be a CUDA device")
-        self.device = torch.device("cuda", dev.index if dev.index is not None else torch.cuda.current_device())
+        self.device = _lib.cuda_device(device)
         self.cfg = cfg if cfg is not None else default_config(task)
         self.n = int(n_envs)
         h = C.c_void_p()
@@ -98,69 +91,73 @@ class QuadXSim:
         except Exception:
             pass
 
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-
-    @staticmethod
-    def _dtype_code(t: torch.Tensor) -> int:
-        if t.dtype == torch.float32:
-            return QX_OBS_F32
-        if t.dtype == torch.bfloat16:
-            return QX_OBS_BF16
-        raise TypeError("obs buffer must be float32 or bfloat16")
-
-    def _check(self, t: torch.Tensor, shape: Sequence[int], dtype: torch.dtype, name: str) -> None:
-        if t.device != self.device or t.dtype != dtype or tuple(t.shape) != tuple(shape) or not t.is_contiguous():
-            raise ValueError(f"{name}: expected contiguous {dtype} {tuple(shape)} on {self.device}, got {t.dtype} {tuple(t.shape)} on {t.device}")
+    def _obs_layout(self, obs: torch.Tensor | None) -> tuple[int, int]:
+        if obs is None:
+            return 0, QX_OBS_F32
+        if obs.device != self.device or obs.dim() != 2 or obs.shape[0] != self.n or obs.stride(1) != 1 or obs.shape[1] < self.obs_dim:
+            raise ValueError("obs: expected [n_envs, >=obs_dim] with unit inner stride on the sim device")
+        if obs.dtype not in (torch.float32, torch.bfloat16):
+            raise TypeError("obs buffer must be float32 or bfloat16")
+        return obs.stride(0), QX_OBS_F32 if obs.dtype == torch.float32 else QX_OBS_BF16
 
     # -- device API ----------------------------------------------------------------
     def reset(self, obs: torch.Tensor | None = None, mask: torch.Tensor | None = None) -> None:
         """qx_reset: obs [n, >=obs_dim] f32/bf16 (row stride = obs.stride(0)), mask u8/bool [n]."""
-        stride, code = 0, QX_OBS_F32
-        if obs is not None:
-            if obs.device != self.device or obs.dim() != 2 or obs.shape[0] != self.n or obs.stride(1) != 1:
-                raise ValueError("obs: expected [n_envs, >=obs_dim] with unit inner stride on the sim device")
-            stride, code = obs.stride(0), self._dtype_code(obs)
+        stride, code = self._obs_layout(obs)
         if mask is not None:
             if mask.dtype == torch.bool:
                 mask = mask.view(torch.uint8)
-            self._check(mask, (self.n,), torch.uint8, "mask")
-        check(self.lib.qx_reset(self._h, _ptr(mask), _ptr(obs), code, stride, self._stream()))
+            expect(mask, "mask", dtype=torch.uint8, device=self.device, shape=(self.n,))
+        check(self.lib.qx_reset(self._h, ptr(mask), ptr(obs), code, stride, stream(self.device)))
+
+    def _step_args(self, actions, obs, reward, terminated, truncated, terminal_obs) -> tuple:
+        expect(actions, "actions", dtype=torch.float32, device=self.device, shape=(self.n, self.act_dim))
+        expect(reward, "reward", dtype=torch.float32, device=self.device, shape=(self.n,))
+        expect(terminated, "terminated", dtype=torch.uint8, device=self.device, shape=(self.n,))
+        expect(truncated, "truncated", dtype=torch.uint8, device=self.device, shape=(self.n,))
+        stride, code = self._obs_layout(obs)
+        if terminal_obs is not None:
+            expect(terminal_obs, "terminal_obs", dtype=torch.float32, device=self.device, shape=(self.n, self.obs_dim))
+        return (self._h, ptr(actions), ptr(obs), code, stride, ptr(reward), ptr(terminated), ptr(truncated), ptr(terminal_obs),
+                stream(self.device))
 
     def step(self, actions: torch.Tensor, obs: torch.Tensor | None, reward: torch.Tensor, terminated: torch.Tensor,
              truncated: torch.Tensor, terminal_obs: torch.Tensor | None = None, split: bool = False) -> None:
         """qx_step on the current stream; all buffers are caller-owned device tensors.  ``split=True`` issues the two
-        halves qx_step_begin + qx_step_end (the deferred reset-queue path the PPO rollout uses) instead of qx_step, which
+        halves step_begin + step_end (the deferred reset-queue path the PPO rollout uses) instead of qx_step, which
         resets finished envs inside the step launch for small batches."""
-        self._check(actions, (self.n, self.act_dim), torch.float32, "actions")
-        self._check(reward, (self.n,), torch.float32, "reward")
-        self._check(terminated, (self.n,), torch.uint8, "terminated")
-        self._check(truncated, (self.n,), torch.uint8, "truncated")
-        stride, code = 0, QX_OBS_F32
-        if obs is not None:
-            if obs.device != self.device or obs.dim() != 2 or obs.shape[0] != self.n or obs.stride(1) != 1 or obs.shape[1] < self.obs_dim:
-                raise ValueError("obs: expected [n_envs, >=obs_dim] with unit inner stride on the sim device")
-            stride, code = obs.stride(0), self._dtype_code(obs)
-        if terminal_obs is not None:
-            self._check(terminal_obs, (self.n, self.obs_dim), torch.float32, "terminal_obs")
         if split:
-            check(self.lib.qx_step_begin(self._h, _ptr(actions), _ptr(obs), code, stride, _ptr(reward), _ptr(terminated),
-                                         _ptr(truncated), _ptr(terminal_obs), self._stream()))
-            check(self.lib.qx_step_end(self._h, _ptr(obs), code, stride, self._stream()))
+            self.step_begin(actions, obs, reward, terminated, truncated, terminal_obs)
+            self.step_end(obs)
             return
-        check(self.lib.qx_step(self._h, _ptr(actions), _ptr(obs), code, stride, _ptr(reward), _ptr(terminated),
-                               _ptr(truncated), _ptr(terminal_obs), self._stream()))
+        check(self.lib.qx_step(*self._step_args(actions, obs, reward, terminated, truncated, terminal_obs)))
+
+    def step_begin(self, actions: torch.Tensor, obs: torch.Tensor | None, reward: torch.Tensor, terminated: torch.Tensor,
+                   truncated: torch.Tensor, terminal_obs: torch.Tensor | None = None) -> None:
+        """qx_step_begin, the first half of step(split=True): the step, with the finished envs queued (done_queue) for step_end."""
+        check(self.lib.qx_step_begin(*self._step_args(actions, obs, reward, terminated, truncated, terminal_obs)))
+
+    def step_end(self, obs: torch.Tensor | None) -> None:
+        """qx_step_end: re-create the envs step_begin queued and write their first observation."""
+        stride, code = self._obs_layout(obs)
+        check(self.lib.qx_step_end(self._h, ptr(obs), code, stride, stream(self.device)))
+
+    def done_queue(self) -> tuple[C.c_void_p, C.c_void_p]:
+        """qx_done_queue: the fixed device addresses of (count, env indices) of the envs the last step_begin queued."""
+        cnt, idx = C.c_void_p(), C.c_void_p()
+        check(self.lib.qx_done_queue(self._h, C.byref(cnt), C.byref(idx)))
+        return cnt, idx
 
     def step_k(self, actions: torch.Tensor, obs: torch.Tensor | None, reward: torch.Tensor, terminated: torch.Tensor,
                truncated: torch.Tensor) -> None:
         k = actions.shape[0]
-        self._check(actions, (k, self.n, self.act_dim), torch.float32, "actions")
+        expect(actions, "actions", dtype=torch.float32, device=self.device, shape=(k, self.n, self.act_dim))
         if obs is not None:
-            self._check(obs, (k, self.n, self.obs_dim), torch.float32, "obs")
-        self._check(reward, (k, self.n), torch.float32, "reward")
-        self._check(terminated, (k, self.n), torch.uint8, "terminated")
-        self._check(truncated, (k, self.n), torch.uint8, "truncated")
-        check(self.lib.qx_step_k(self._h, k, _ptr(actions), _ptr(obs), _ptr(reward), _ptr(terminated), _ptr(truncated), self._stream()))
+            expect(obs, "obs", dtype=torch.float32, device=self.device, shape=(k, self.n, self.obs_dim))
+        expect(reward, "reward", dtype=torch.float32, device=self.device, shape=(k, self.n))
+        expect(terminated, "terminated", dtype=torch.uint8, device=self.device, shape=(k, self.n))
+        expect(truncated, "truncated", dtype=torch.uint8, device=self.device, shape=(k, self.n))
+        check(self.lib.qx_step_k(self._h, k, ptr(actions), ptr(obs), ptr(reward), ptr(terminated), ptr(truncated), stream(self.device)))
 
     def render(self, env_idx: torch.Tensor | Sequence[int] | None = None, fmt: str = "rgba", out: torch.Tensor | None = None) -> torch.Tensor:
         """qx_render: the FPV camera frames of the envs' current poses (those the last observation's camera columns were
@@ -173,7 +170,7 @@ class QuadXSim:
             raise ValueError(f"fmt must be 'rgba' or 'mask', got {fmt!r}")
         if env_idx is not None:
             if isinstance(env_idx, torch.Tensor):
-                self._check(env_idx, (env_idx.numel(),), torch.int32, "env_idx")
+                expect(env_idx, "env_idx", dtype=torch.int32, device=self.device, shape=(env_idx.numel(),))
             else:
                 env_idx = torch.tensor(list(env_idx), dtype=torch.int32, device=self.device)
         m = self.n if env_idx is None else env_idx.numel()
@@ -182,8 +179,8 @@ class QuadXSim:
         if out is None:
             out = torch.empty(shape, dtype=torch.uint8, device=self.device)
         else:
-            self._check(out, shape, torch.uint8, "out")
-        check(self.lib.qx_render(self._h, _ptr(env_idx), m, code, _ptr(out), self._stream()))
+            expect(out, "out", dtype=torch.uint8, device=self.device, shape=shape)
+        check(self.lib.qx_render(self._h, ptr(env_idx), m, code, ptr(out), stream(self.device)))
         return out
 
     def episode_record(self, ret: torch.Tensor, length: torch.Tensor, end: torch.Tensor, n_closed: torch.Tensor) -> None:
@@ -191,11 +188,11 @@ class QuadXSim:
         of envs whose episode has ended are closed with the episode's return (f32 [n]), length (int32 [n]) and flags word
         (int32 [n], the bits of qx_get_flags, never 0 once closed); n_closed (int32 [1]) counts the closed records.  Zero
         `end` and `n_closed` before the first step of an evaluation."""
-        self._check(ret, (self.n,), torch.float32, "ret")
-        self._check(length, (self.n,), torch.int32, "length")
-        self._check(end, (self.n,), torch.int32, "end")  # u32 words on the device; the flag bits stay below bit 31
-        self._check(n_closed, (1,), torch.int32, "n_closed")
-        check(self.lib.qx_episode_record(self._h, _ptr(ret), _ptr(length), _ptr(end), _ptr(n_closed), self._stream()))
+        expect(ret, "ret", dtype=torch.float32, device=self.device, shape=(self.n,))
+        expect(length, "length", dtype=torch.int32, device=self.device, shape=(self.n,))
+        expect(end, "end", dtype=torch.int32, device=self.device, shape=(self.n,))  # u32 words on the device; the flag bits stay below bit 31
+        expect(n_closed, "n_closed", dtype=torch.int32, device=self.device, shape=(1,))
+        check(self.lib.qx_episode_record(self._h, ptr(ret), ptr(length), ptr(end), ptr(n_closed), stream(self.device)))
 
     # -- host API ----------------------------------------------------------------
     def reset_host(self, mask: np.ndarray | None = None) -> np.ndarray:
@@ -223,13 +220,12 @@ class QuadXSim:
                           truncated: torch.Tensor) -> None:
         """qx_step_host_ex on caller-owned CPU tensors (pinned ones are read / written in place by the copy engines):
         `obs` is float32 or bfloat16 [n, obs_dim] -- bfloat16 halves the bytes of the device-to-host copy that bounds this call."""
-        for t, shape, dt, name in ((actions, (self.n, self.act_dim), (torch.float32,), "actions"), (obs, (self.n, self.obs_dim), (torch.float32, torch.bfloat16), "obs"),
-                                   (reward, (self.n,), (torch.float32,), "reward"), (terminated, (self.n,), (torch.uint8,), "terminated"),
-                                   (truncated, (self.n,), (torch.uint8,), "truncated")):
-            if t.device.type != "cpu" or tuple(t.shape) != shape or t.dtype not in dt or not t.is_contiguous():
-                raise ValueError(f"{name}: expected a contiguous CPU tensor {shape} of {dt}, got {tuple(t.shape)} {t.dtype} on {t.device}")
-        check(self.lib.qx_step_host_ex(self._h, _ptr(actions), _ptr(obs), 1 if obs.dtype == torch.bfloat16 else 0, _ptr(reward), _ptr(terminated),
-                                       _ptr(truncated), None))
+        for t, shape, dt, name in ((actions, (self.n, self.act_dim), torch.float32, "actions"), (obs, (self.n, self.obs_dim), (torch.float32, torch.bfloat16), "obs"),
+                                   (reward, (self.n,), torch.float32, "reward"), (terminated, (self.n,), torch.uint8, "terminated"),
+                                   (truncated, (self.n,), torch.uint8, "truncated")):
+            expect(t, name, dtype=dt, device=torch.device("cpu"), shape=shape)
+        check(self.lib.qx_step_host_ex(self._h, ptr(actions), ptr(obs), 1 if obs.dtype == torch.bfloat16 else 0, ptr(reward), ptr(terminated),
+                                       ptr(truncated), None))
 
     @property
     def state_fields(self) -> list[str]:

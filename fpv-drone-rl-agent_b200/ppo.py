@@ -25,18 +25,21 @@ import torch.distributed as dist
 from torch import nn
 
 from . import _lib
-from ._lib import PpoPolicy, check
+from ._lib import PpoPolicy, QxConfig, check, default_config, expect, ptr, stream
 from .hover_env import QuadXSim
 
 HID, IN_PAD, HEAD_PAD = 128, 32, 16
 
 
-def _p(t: torch.Tensor | None):
-    return None if t is None else C.c_void_p(t.data_ptr())
-
-
-def _stream(dev):
-    return C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+def _capture(body, device) -> torch.cuda.CUDAGraph:
+    """Capture `body` into a CUDA graph on a fresh side stream forked from, and joined back into, the current stream."""
+    side = torch.cuda.Stream(device=device)
+    side.wait_stream(torch.cuda.current_stream(device))
+    g = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(g, stream=side):
+        body()
+    torch.cuda.current_stream(device).wait_stream(side)
+    return g
 
 
 class ActorCritic(nn.Module):
@@ -178,7 +181,7 @@ class PackedPolicy:
     """bf16 copy of an ``ActorCritic`` in the layout of ``struct PpoPolicy``."""
 
     def __init__(self, model: ActorCritic, device):
-        self.model, self.device = model, torch.device(device)
+        self.model, self.device = model, _lib.cuda_device(device)
         d = self.device
         self.w1 = torch.zeros(2 * HID, IN_PAD, dtype=torch.bfloat16, device=d)
         self.w2p = torch.zeros(HID, HID, dtype=torch.bfloat16, device=d)
@@ -188,7 +191,6 @@ class PackedPolicy:
         self.b2 = torch.zeros(2 * HID, device=d)
         self.b3 = torch.zeros(HEAD_PAD, device=d)
         self.log_std = torch.zeros(4, device=d)
-        self.device = self.w1.device  # with its index ("cuda" -> "cuda:<current>"): what the outputs of policy_forward must be on
         self.struct = PpoPolicy(self.w1.data_ptr(), self.w2p.data_ptr(), self.w2v.data_ptr(), self.w3.data_ptr(), self.b1.data_ptr(),
                                 self.b2.data_ptr(), self.b3.data_ptr(), self.log_std.data_ptr(), model.obs_dim, model.act_dim)
         self.refresh()
@@ -216,8 +218,8 @@ class RunningStats:
     """VecNormalize ``RunningMeanStd`` kept on the device: {mean[dim], var[dim], count} in fp64."""
 
     def __init__(self, dim: int, device, eps: float = 1e-8):
-        self.dim, self.eps, self.device = dim, eps, torch.device(device)
         self.stats = torch.zeros(2 * dim + 1, dtype=torch.float64, device=device)
+        self.dim, self.eps, self.device = dim, eps, self.stats.device  # device with its index; CPU statistics serve export / gloo tests
         self.stats[dim:2 * dim] = 1.0
         self.stats[2 * dim] = 1e-4  # RunningMeanStd(epsilon=1e-4)
         self.mean = torch.zeros(dim, device=device)
@@ -228,8 +230,8 @@ class RunningStats:
         """Merge the rows of x; the refreshed fp32 (mean, inv_std) go to `out` instead of self.mean / self.inv_std when given."""
         assert x.dtype == torch.float32 and x.dim() == 2 and x.shape[1] >= self.dim and x.stride(1) == 1
         mean, inv_std = out if out is not None else (self.mean, self.inv_std)
-        check(_lib.lib().ppo_running_stats_update(_p(x), x.stride(0), x.shape[0], self.dim, _p(self.stats), self.eps, _p(mean),
-                                                  _p(inv_std), _p(self.scratch), _stream(self.device)))
+        check(_lib.lib().ppo_running_stats_update(ptr(x), x.stride(0), x.shape[0], self.dim, ptr(self.stats), self.eps, ptr(mean),
+                                                  ptr(inv_std), ptr(self.scratch), stream(self.device)))
 
     def state_dict(self):
         return {"stats": self.stats.clone(), "mean": self.mean.clone(), "inv_std": self.inv_std.clone()}
@@ -265,25 +267,23 @@ def policy_forward(pol: PackedPolicy, obs: torch.Tensor, *, obs_stats: RunningSt
     with fused_stats, one launch with the merge inside the policy kernel."""
     n = obs.shape[0]
     assert obs.dtype == torch.float32 and obs.stride(1) == 1
-    # the kernel writes dense [n, act_dim], [n] and [n, obs_dim] arrays from the base pointer: anything else would be written wrongly
     od, ad, dev = pol.model.obs_dim, pol.model.act_dim, pol.device
     for name, t, numel in (("actions", actions, n * ad), ("env_actions", env_actions, n * ad), ("values", values, n),
                            ("log_probs", log_probs, n), ("obs_norm", obs_norm, n * od)):
-        if t is not None and (t.dtype != torch.float32 or t.device != dev or not t.is_contiguous() or t.numel() != numel):
-            raise ValueError(f"policy_forward: {name} must be a contiguous float32 tensor of {numel} elements on {dev}, "
-                             f"got {tuple(t.shape)} {t.dtype} on {t.device} (contiguous: {t.is_contiguous()})")
+        if t is not None:
+            expect(t, name, dtype=torch.float32, device=dev, numel=numel)
     mean, inv_std = norm if norm is not None else ((obs_stats.mean, obs_stats.inv_std) if obs_stats else (None, None))
     if update_stats:
         assert obs_stats is not None and mean is not None
-        check(_lib.lib().ppo_policy_forward_stats(C.byref(pol.struct), _p(obs), obs.stride(0), n, _p(obs_stats.stats), obs_stats.eps,
-                                                  _p(obs_stats.scratch), _p(mean), _p(inv_std), obs_clip, seed, row0, step, _p(step_base),
-                                                  int(deterministic), _p(actions), _p(env_actions), _p(values), _p(log_probs), _p(obs_norm),
-                                                  int(fused_stats), _stream(pol.device)))
+        check(_lib.lib().ppo_policy_forward_stats(C.byref(pol.struct), ptr(obs), obs.stride(0), n, ptr(obs_stats.stats), obs_stats.eps,
+                                                  ptr(obs_stats.scratch), ptr(mean), ptr(inv_std), obs_clip, seed, row0, step, ptr(step_base),
+                                                  int(deterministic), ptr(actions), ptr(env_actions), ptr(values), ptr(log_probs), ptr(obs_norm),
+                                                  int(fused_stats), stream(pol.device)))
         return
-    check(_lib.lib().ppo_policy_forward(C.byref(pol.struct), _p(obs), obs.stride(0), n, _p(mean),
-                                        _p(inv_std), obs_clip, seed, row0, step, _p(step_base),
-                                        int(deterministic), _p(actions), _p(env_actions), _p(values), _p(log_probs), _p(obs_norm),
-                                        _stream(pol.device)))
+    check(_lib.lib().ppo_policy_forward(C.byref(pol.struct), ptr(obs), obs.stride(0), n, ptr(mean),
+                                        ptr(inv_std), obs_clip, seed, row0, step, ptr(step_base),
+                                        int(deterministic), ptr(actions), ptr(env_actions), ptr(values), ptr(log_probs), ptr(obs_norm),
+                                        stream(pol.device)))
 
 
 F_TERMINATED, F_TRUNCATED, F_OUT_OF_BOUNDS, F_ON_FLOOR = 2, 4, 8, 16  # bits of the flags word (qx_get_flags)
@@ -305,8 +305,6 @@ class PolicyEvaluator:
 
     def __init__(self, policy: PackedPolicy, obs_stats: RunningStats | None, env_cfg=None, n_episodes: int = 4096, seed: int = 0,
                  task: int = 0, obs_clip: float = 10.0, device=None, chunk: int = 32, use_cuda_graph: bool = True):
-        from ._lib import QxConfig, default_config
-
         if n_episodes <= 0 or chunk <= 0:
             raise ValueError("n_episodes and chunk must be positive")
         cfg = default_config(task) if env_cfg is None else QxConfig.from_buffer_copy(env_cfg)
@@ -353,14 +351,7 @@ class PolicyEvaluator:
             self._chunk()
             return
         if self._graph is None:
-            st = torch.cuda.Stream(device=self.device)
-            st.wait_stream(torch.cuda.current_stream(self.device))
-            with torch.cuda.stream(st):
-                g = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(g, stream=st):
-                    self._chunk()
-            torch.cuda.current_stream(self.device).wait_stream(st)
-            self._graph = g
+            self._graph = _capture(self._chunk, self.device)
         self._graph.replay()
 
     def evaluate(self) -> tuple[dict, dict]:
@@ -411,8 +402,37 @@ def evaluate_policy(policy: PackedPolicy, obs_stats: RunningStats | None, env_cf
 def gae(rewards, values, dones, last_values, gamma: float, lam: float, advantages, returns) -> None:
     """``RolloutBuffer.compute_returns_and_advantage`` (ppo_gae); all [T, n] contiguous."""
     T, n = rewards.shape
-    check(_lib.lib().ppo_gae(_p(rewards), _p(values), _p(dones), _p(last_values), T, n, gamma, lam, _p(advantages), _p(returns),
-                             _stream(rewards.device)))
+    check(_lib.lib().ppo_gae(ptr(rewards), ptr(values), ptr(dones), ptr(last_values), T, n, gamma, lam, ptr(advantages), ptr(returns),
+                             stream(rewards.device)))
+
+
+def bootstrap_truncated(pol: PackedPolicy, terminal_obs, norm: tuple | None, obs_clip: float, queue: tuple, terminated, truncated,
+                        gamma: float, rewards, *, first: bool = False) -> None:
+    """SB3's time-limit bootstrap (ppo_bootstrap_truncated): rewards[i] += gamma * V(terminal_obs[i]) for the truncated, not terminated
+    envs of the done queue (QuadXSim.done_queue()).  first: rewards[i] = gamma * V(...) instead, for reward_normalize(add=True)."""
+    n, dev = terminal_obs.shape[0], pol.device
+    expect(terminal_obs, "terminal_obs", dtype=torch.float32, device=dev, shape=(n, pol.model.obs_dim))
+    expect(terminated, "terminated", dtype=torch.uint8, device=dev, numel=n)
+    expect(truncated, "truncated", dtype=torch.uint8, device=dev, numel=n)
+    expect(rewards, "rewards", dtype=torch.float32, device=dev, numel=n)
+    mean, inv_std = norm if norm is not None else (None, None)
+    fn = _lib.lib().ppo_bootstrap_truncated_first if first else _lib.lib().ppo_bootstrap_truncated
+    check(fn(C.byref(pol.struct), ptr(terminal_obs), terminal_obs.stride(0), n, ptr(mean), ptr(inv_std), obs_clip, queue[0], queue[1],
+             ptr(terminated), ptr(truncated), gamma, ptr(rewards), stream(dev)))
+
+
+def reward_normalize(raw_reward, terminated, truncated, returns_acc, ret_stats: RunningStats, gamma: float, clip: float, rewards, dones,
+                     *, add: bool = False) -> None:
+    """VecNormalize's reward path (ppo_reward_normalize): returns_acc = gamma * returns_acc + raw_reward into ret_stats, rewards =
+    clip(raw_reward / std), dones = terminated | truncated.  add: plus what bootstrap_truncated(first=True) stored in rewards."""
+    n, dev = raw_reward.shape[0], ret_stats.device
+    for name, t, dtype in (("raw_reward", raw_reward, torch.float32), ("terminated", terminated, torch.uint8), ("truncated", truncated, torch.uint8),
+                           ("returns_acc", returns_acc, torch.float32), ("rewards", rewards, torch.float32), ("dones", dones, torch.uint8)):
+        expect(t, name, dtype=dtype, device=dev, numel=n)
+    expect(ret_stats.stats, "ret_stats", dtype=torch.float64, device=dev, numel=3)
+    fn = _lib.lib().ppo_reward_normalize_add if add else _lib.lib().ppo_reward_normalize
+    check(fn(ptr(raw_reward), ptr(terminated), ptr(truncated), ptr(returns_acc), n, gamma, clip, ret_stats.eps, ptr(ret_stats.stats),
+             ptr(rewards), ptr(dones), ptr(ret_stats.scratch), stream(dev)))
 
 
 def allreduce_gradients(params, world: int) -> None:
@@ -490,7 +510,6 @@ class RolloutEngine:
 
     def __init__(self, sim: QuadXSim, policy: PackedPolicy, cfg: PPOConfig, row0: int = 0):
         self.sim, self.pol, self.cfg = sim, policy, cfg
-        self.lib = _lib.lib()
         n, T, d = sim.n, cfg.n_steps, sim.device
         od, ad = sim.obs_dim, sim.act_dim
         self.n, self.T, self.device, self.row0 = n, T, d, row0
@@ -514,9 +533,7 @@ class RolloutEngine:
         self.obs_stats = RunningStats(od, d)
         self.ret_stats = RunningStats(1, d)
         self.step_base = torch.zeros(1, dtype=torch.int64, device=d)
-        cnt, idx = C.c_void_p(), C.c_void_p()
-        check(self.lib.qx_done_queue(sim._h, C.byref(cnt), C.byref(idx)))
-        self._q_count, self._q_idx = cnt, idx
+        self._done_queue = sim.done_queue()
         self._graph = None
         self._side = torch.cuda.Stream(device=d)
         self._snap_mean = torch.zeros(2, od, **f)  # fp32 (mean, inv_std) of the observation statistics, one pair per step parity
@@ -532,7 +549,7 @@ class RolloutEngine:
     # observation statistics of step t, so (a) main joins it before the env step of t + 1 overwrites those, and (b) the fp32
     # (mean, inv_std) of step t live in the buffer pair t & 1, which the statistics update of step t + 1 does not touch.
     def _step(self, t: int) -> None:
-        cfg, sim, L, s = self.cfg, self.sim, self.lib, _stream(self.device)
+        cfg, sim = self.cfg, self.sim
         stats = self.obs_stats if cfg.norm_obs else None
         norm = (self._snap_mean[t & 1], self._snap_inv[t & 1]) if cfg.norm_obs else None
         chain = cfg.norm_obs and (cfg.fuse_obs_stats or cfg.chain_obs_stats)
@@ -544,31 +561,26 @@ class RolloutEngine:
         main = torch.cuda.current_stream(self.device)
         if t > 0:
             main.wait_stream(self._side)  # join the side branch of step t - 1 (the rollout ends with a join, so there is none at t = 0)
-        check(L.qx_step_begin(sim._h, _p(self.env_actions), _p(self.cur_obs), 0, self.cur_obs.stride(0), _p(self.raw_reward), _p(self.te),
-                              _p(self.tr), _p(self.terminal_obs), s))
+        sim.step_begin(self.env_actions, self.cur_obs, self.raw_reward, self.te, self.tr, self.terminal_obs)
         self._side.wait_stream(main)  # fork
         with torch.cuda.stream(self._side):
-            ss = _stream(self.device)
-            boot_args = (C.byref(self.pol.struct), _p(self.terminal_obs), self.terminal_obs.stride(0), self.n,
-                         _p(norm[0]) if norm else None, _p(norm[1]) if norm else None, cfg.clip_obs,
-                         self._q_count, self._q_idx, _p(self.te), _p(self.tr), cfg.gamma, _p(self.rewards[t]), ss)
-            norm_args = (_p(self.raw_reward), _p(self.te), _p(self.tr), _p(self.returns_acc), self.n, cfg.gamma, cfg.clip_reward,
-                         self.ret_stats.eps, _p(self.ret_stats.stats), _p(self.rewards[t]), _p(self.dones[t]), _p(self.ret_stats.scratch), ss)
+            boot_args = (self.pol, self.terminal_obs, norm, cfg.clip_obs, self._done_queue, self.te, self.tr, cfg.gamma, self.rewards[t])
+            norm_args = (self.raw_reward, self.te, self.tr, self.returns_acc, self.ret_stats, cfg.gamma, cfg.clip_reward, self.rewards[t], self.dones[t])
             boot_first = cfg.bootstrap_first if cfg.bootstrap_first is not None else (sim.obs_dim != 20)  # yaw: 12-D observation
             if cfg.norm_reward and boot_first:
                 # the bootstrap launch needs a whole SM's shared memory per CTA even to find the done queue empty: issued first it runs
                 # while the main branch is still in the reset / statistics launches, not after the policy CTAs have taken the SMs
-                check(L.ppo_bootstrap_truncated_first(*boot_args))
-                check(L.ppo_reward_normalize_add(*norm_args))
+                bootstrap_truncated(*boot_args, first=True)
+                reward_normalize(*norm_args, add=True)
             else:
                 if cfg.norm_reward:
-                    check(L.ppo_reward_normalize(*norm_args))
+                    reward_normalize(*norm_args)
                 else:
                     self.rewards[t].copy_(self.raw_reward)
                     torch.bitwise_or(self.te, self.tr, out=self.dones[t])
                 # SB3: rewards[idx] += gamma * V(terminal_obs) when the time limit, not the task, ended the episode
-                check(L.ppo_bootstrap_truncated(*boot_args))
-        check(L.qx_step_end(sim._h, _p(self.cur_obs), 0, self.cur_obs.stride(0), s))
+                bootstrap_truncated(*boot_args)
+        sim.step_end(self.cur_obs)
 
     def _rollout_body(self) -> None:
         for t in range(self.T):
@@ -588,14 +600,7 @@ class RolloutEngine:
             self._rollout_body()
             return
         if self._graph is None:
-            st = torch.cuda.Stream(device=self.device)
-            st.wait_stream(torch.cuda.current_stream(self.device))
-            with torch.cuda.stream(st):
-                g = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(g, stream=st):
-                    self._rollout_body()
-            torch.cuda.current_stream(self.device).wait_stream(st)
-            self._graph = g
+            self._graph = _capture(self._rollout_body, self.device)
         self._graph.replay()
 
     @property
@@ -620,9 +625,7 @@ class FusedUpdater:
     minibatches are sets of 128-row tiles of the rollout buffers (a random permutation of the tiles per epoch)."""
 
     def __init__(self, model: ActorCritic, packed: PackedPolicy, cfg: "PPOConfig", device, world: int = 1):
-        self.model, self.packed, self.cfg, self.device, self.world = model, packed, cfg, torch.device(device), world
-        if self.device.type == "cuda" and self.device.index is None:
-            self.device = torch.device("cuda", torch.cuda.current_device())
+        self.model, self.packed, self.cfg, self.device, self.world = model, packed, cfg, _lib.cuda_device(device), world
         self.lib = _lib.lib()
         od, ad = model.obs_dim, model.act_dim
         self.n_params = int(self.lib.ppo_update_num_params(od, ad))
@@ -640,27 +643,28 @@ class FusedUpdater:
         self.exp_avg_sq = torch.zeros(self.n_params, **f)
         self.loss_stats = torch.zeros(8, **f)
         self.workspace = torch.zeros(int(self.lib.ppo_update_workspace_bytes(od, ad)) // 4 + 4, **f)  # zero-filled once
+        self._all_tiles = torch.arange((cfg.n_steps * cfg.n_envs + 127) // 128, dtype=torch.int32, device=self.device)  # recompute_logp
         packed.refresh()
 
     def gradient(self, ro: "RolloutEngine", tiles: torch.Tensor, normalize_adv: bool = True) -> torch.Tensor:
         """Mean gradient of the PPO loss over the minibatch `tiles` (int32 device tensor of 128-row tile indices)."""
         cfg, N = self.cfg, ro.T * ro.n
         assert tiles.dtype == torch.int32 and tiles.device == self.device and tiles.is_contiguous()
-        check(self.lib.ppo_update_minibatch(C.byref(self.packed.struct), _p(ro.obs), _p(ro.actions), _p(ro.log_probs), _p(ro.advantages),
-                                            _p(ro.returns), _p(tiles), tiles.numel(), N, cfg.clip_range, cfg.vf_coef, cfg.ent_coef,
-                                            int(normalize_adv), _p(self.grad), _p(self.loss_stats), _p(self.workspace), _stream(self.device)))
+        check(self.lib.ppo_update_minibatch(C.byref(self.packed.struct), ptr(ro.obs), ptr(ro.actions), ptr(ro.log_probs), ptr(ro.advantages),
+                                            ptr(ro.returns), ptr(tiles), tiles.numel(), N, cfg.clip_range, cfg.vf_coef, cfg.ent_coef,
+                                            int(normalize_adv), ptr(self.grad), ptr(self.loss_stats), ptr(self.workspace), stream(self.device)))
         return self.grad[:self.n_params]
 
     def apply(self) -> None:
         """All-reduce (world > 1), clip, Adam, re-pack."""
-        cfg, s = self.cfg, _stream(self.device)
+        cfg, s = self.cfg, stream(self.device)
         scale = 1.0
         if self.world > 1:
             dist.all_reduce(self.grad)
             scale = 1.0 / self.world
-            check(self.lib.ppo_update_grad_norm(_p(self.grad), self.n_params, scale, _p(self.workspace), s))
-        check(self.lib.ppo_update_adam(_p(self.flat), _p(self.grad), _p(self.exp_avg), _p(self.exp_avg_sq), self.n_params, cfg.learning_rate,
-                                       0.9, 0.999, 1e-5, cfg.max_grad_norm, scale, C.byref(self.packed.struct), _p(self.workspace), s))
+            check(self.lib.ppo_update_grad_norm(ptr(self.grad), self.n_params, scale, ptr(self.workspace), s))
+        check(self.lib.ppo_update_adam(ptr(self.flat), ptr(self.grad), ptr(self.exp_avg), ptr(self.exp_avg_sq), self.n_params, cfg.learning_rate,
+                                       0.9, 0.999, 1e-5, cfg.max_grad_norm, scale, C.byref(self.packed.struct), ptr(self.workspace), s))
 
     def step(self, ro: "RolloutEngine", tiles: torch.Tensor) -> None:
         self.gradient(ro, tiles)
@@ -668,34 +672,32 @@ class FusedUpdater:
 
     def recompute_logp(self, ro: "RolloutEngine") -> None:
         """Overwrite the rollout's log-probs with the update kernel's own forward pass (ppo_update_recompute_logp)."""
-        N = ro.T * ro.n
-        n_tiles = (N + 127) // 128
-        if getattr(self, "_all_tiles", None) is None or self._all_tiles.numel() != n_tiles:
-            self._all_tiles = torch.arange(n_tiles, dtype=torch.int32, device=self.device)
-        check(self.lib.ppo_update_recompute_logp(C.byref(self.packed.struct), _p(ro.obs), _p(ro.actions), _p(self._all_tiles), n_tiles, N,
-                                                 _p(ro.log_probs), _p(self.workspace), _stream(self.device)))
+        N, n_tiles = ro.T * ro.n, self._all_tiles.numel()
+        assert (N + 127) // 128 == n_tiles, "the rollout is not the n_steps x n_envs of the updater's config"
+        check(self.lib.ppo_update_recompute_logp(C.byref(self.packed.struct), ptr(ro.obs), ptr(ro.actions), ptr(self._all_tiles), n_tiles, N,
+                                                 ptr(ro.log_probs), ptr(self.workspace), stream(self.device)))
 
     def arm_kl_stop(self, target_kl: float) -> None:
         """(Re-)arm SB3's target_kl early stop on the device (0 = off) and clear its latch: call once per PPO.train."""
-        check(self.lib.ppo_update_kl_stop(_p(self.workspace), float(target_kl), None, None, _stream(self.device)))
+        check(self.lib.ppo_update_kl_stop(ptr(self.workspace), float(target_kl), None, None, stream(self.device)))
 
     def kl_stopped(self) -> tuple[bool, int]:
         """(latched, optimiser steps skipped since arm_kl_stop)."""
         st, sk = C.c_int32(), C.c_int32()
-        check(self.lib.ppo_update_kl_stop(_p(self.workspace), -1.0, C.byref(st), C.byref(sk), _stream(self.device)))
+        check(self.lib.ppo_update_kl_stop(ptr(self.workspace), -1.0, C.byref(st), C.byref(sk), stream(self.device)))
         return bool(st.value), sk.value
 
     def set_log_std_floor(self, floor: float | None) -> None:
-        check(self.lib.ppo_update_set_log_std_floor(_p(self.workspace), 0 if floor is None else 1, 0.0 if floor is None else float(floor), _stream(self.device)))
+        check(self.lib.ppo_update_set_log_std_floor(ptr(self.workspace), 0 if floor is None else 1, 0.0 if floor is None else float(floor), stream(self.device)))
 
     def set_lr_scale(self, scale: float) -> None:
         """Learning-rate schedule: later optimiser steps (graph replays included) use learning_rate * scale."""
-        check(self.lib.ppo_update_set_lr_scale(_p(self.workspace), float(scale), _stream(self.device)))
+        check(self.lib.ppo_update_set_lr_scale(ptr(self.workspace), float(scale), stream(self.device)))
 
     @property
     def adam_steps(self) -> int:
         out = C.c_int64()
-        check(self.lib.ppo_update_step_count(_p(self.workspace), -1, C.byref(out), _stream(self.device)))
+        check(self.lib.ppo_update_step_count(ptr(self.workspace), -1, C.byref(out), stream(self.device)))
         return out.value
 
     def state_dict(self) -> dict:
@@ -703,7 +705,7 @@ class FusedUpdater:
 
     def load_state_dict(self, sd: dict) -> None:
         self.flat.copy_(sd["flat"]); self.exp_avg.copy_(sd["exp_avg"]); self.exp_avg_sq.copy_(sd["exp_avg_sq"])
-        check(self.lib.ppo_update_step_count(_p(self.workspace), int(sd["adam_steps"]), None, _stream(self.device)))
+        check(self.lib.ppo_update_step_count(ptr(self.workspace), int(sd["adam_steps"]), None, stream(self.device)))
         self.packed.refresh()
 
 
@@ -713,18 +715,13 @@ class PPOTrainer:
     def __init__(self, cfg: PPOConfig, device=None, env_cfg=None, rank: int = 0, world: int = 1, task: int = 0):
         """task: QX_TASK_HOVER (0, hover.py) or QX_TASK_YAW (1, yaw.py: 12-D obs, 1-D action)."""
         self.cfg, self.rank, self.world = cfg, rank, world
-        dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
-        if dev.type == "cuda" and dev.index is None:  # "cuda" -> "cuda:<current>": tensors report an indexed device
-            dev = torch.device("cuda", torch.cuda.current_device())
-        self.device = dev
+        self.device = dev = _lib.cuda_device(device)
         if cfg.tf32_update:
             torch.backends.cuda.matmul.allow_tf32 = True
         torch.manual_seed(cfg.seed)  # identical initial weights on every rank
         self.model = (ActorCritic(log_std_init=cfg.log_std_init, hidden=cfg.net_arch) if task == 0
                       else ActorCritic(12, 1, log_std_init=cfg.log_std_init, hidden=cfg.net_arch)).to(dev)
         self.packed = PackedPolicy(self.model, dev)
-        from ._lib import default_config
-
         ecfg = env_cfg if env_cfg is not None else default_config(task)
         ecfg.update(auto_reset=1)
         self.sim = QuadXSim(cfg.n_envs, ecfg, seed=cfg.seed, env_id0=shard_env_ids(rank, cfg.n_envs), device=dev, task=task)
@@ -735,14 +732,12 @@ class PPOTrainer:
         self.opt = None if cfg.fused_update else torch.optim.Adam(self.model.parameters(), lr=cfg.learning_rate, eps=1e-5,
                                                                    capturable=bool(cfg.graph_update and world == 1))
         self._epoch_graph = None
+        self._update_graph = None  # (fused_update=False) one torch minibatch step, see _build_update_graph
+        self._perm = torch.zeros_like(self.fused._all_tiles) if self.fused is not None else None  # the epoch's permutation of the tiles
         self.num_timesteps = 0
         self._iteration = 0
-        self._flat_grad = None
         self._evaluator = None  # PolicyEvaluator of evaluate(), built on its first call
         self.gen = torch.Generator(device=dev).manual_seed(cfg.seed + 1000 + rank)
-
-    def _allreduce_grads(self) -> None:
-        allreduce_gradients(self.model.parameters(), self.world)
 
     # one PPO minibatch: loss of SB3's PPO.train (clipped surrogate + vf_coef * MSE - ent_coef * entropy, advantages
     # normalised per minibatch) and the diagnostics it logs; `acc` accumulates [pg, vf, kl, clipfrac, approx_kl_k3]
@@ -768,7 +763,7 @@ class PPOTrainer:
         loss = self._minibatch_loss(idx, acc)
         self.opt.zero_grad(set_to_none=True)
         loss.backward()
-        self._allreduce_grads()
+        allreduce_gradients(self.model.parameters(), self.world)
         torch.nn.utils.clip_grad_norm_(self.model.parameters(), self.cfg.max_grad_norm)
         self.opt.step()
 
@@ -793,16 +788,13 @@ class PPOTrainer:
                 self._step_eager(self._g_idx, self._g_acc)
         torch.cuda.current_stream(self.device).wait_stream(side)
         self.opt.zero_grad(set_to_none=True)
-        g = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(g):
-            self._step_eager(self._g_idx, self._g_acc)
+        self._update_graph = _capture(lambda: self._step_eager(self._g_idx, self._g_acc), self.device)
         with torch.no_grad():  # the warm-up / capture steps must not count as training
             for k, v in self.model.state_dict().items():
                 v.copy_(model_sd[k])
             for st, snap in zip(self.opt.state.values(), opt_snap):
                 for k, v in snap.items():
                     st[k].copy_(v)
-        self._update_graph = g
 
     def _update_fused(self) -> dict:
         """SB3 PPO.train on the hand-written kernels: per epoch a fresh random permutation of the rollout's 128-row tiles,
@@ -813,9 +805,6 @@ class PPOTrainer:
         n_tiles = (N + 127) // 128
         tpm = max(1, min(cfg.batch_size, N) // 128)  # tiles per minibatch
         starts = list(range(0, n_tiles - tpm + 1, tpm)) or [0]
-        if getattr(self, "_perm", None) is None or self._perm.numel() != n_tiles:
-            self._perm = torch.zeros(n_tiles, dtype=torch.int32, device=self.device)
-            self._epoch_graph = None
 
         def epoch_body():
             for s0 in starts:
@@ -840,14 +829,11 @@ class PPOTrainer:
                         fu.step(ro, self._perm[:tpm])  # warm-up outside capture (one-time kernel attributes, NCCL)
                     torch.cuda.current_stream(self.device).wait_stream(side)
                     torch.cuda.synchronize(self.device)
-                    g = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g):
-                        epoch_body()
+                    self._epoch_graph = _capture(epoch_body, self.device)
                     # warm-up and capture must not count as training: restore parameters, moments, step count, statistics
                     fu.load_state_dict({**keep, "adam_steps": steps0})
                     fu.loss_stats.copy_(stats0)
                     fu.arm_kl_stop(dev_kl)
-                    self._epoch_graph = g
                 self._epoch_graph.replay()
             else:
                 epoch_body()
@@ -878,7 +864,7 @@ class PPOTrainer:
         N = ro.T * ro.n
         bs = min(cfg.batch_size, N)
         use_graph = cfg.graph_update and self.world == 1
-        if use_graph and getattr(self, "_update_graph", None) is None:
+        if use_graph and self._update_graph is None:
             self._build_update_graph(bs)
         acc = self._g_acc if use_graph else torch.zeros(5, device=self.device)
         acc.zero_()
@@ -977,7 +963,7 @@ class PPOTrainer:
         if self.fused is not None:
             self.fused.load_state_dict(sd["opt"])
         else:
-            if getattr(self, "_update_graph", None) is not None and self.opt.state:
+            if self._update_graph is not None and self.opt.state:
                 for st, src in zip(self.opt.state.values(), sd["opt"]["state"].values()):  # in place: the graph updates these tensors
                     for k, v in src.items():
                         if torch.is_tensor(v):

@@ -416,6 +416,19 @@ def test_gym_api_conformance(pkg):
     with pytest.raises(ValueError):
         sim.step(torch.zeros(63, 4, device="cuda"), None, torch.zeros(64, device="cuda"), torch.zeros(64, dtype=torch.uint8, device="cuda"),
                  torch.zeros(64, dtype=torch.uint8, device="cuda"))
+    # an observation view with fewer than obs_dim columns: its row stride leaves room for 20, but the view ends before that
+    wide = torch.full((64, 24), 7.0, device="cuda")
+    for narrow in (wide[:, :19], wide[:, :4]):
+        with pytest.raises(ValueError, match="obs"):
+            sim.reset(narrow)
+        with pytest.raises(ValueError, match="obs"):
+            sim.step(torch.zeros(64, 4, device="cuda"), narrow, torch.zeros(64, device="cuda"), torch.zeros(64, dtype=torch.uint8, device="cuda"),
+                     torch.zeros(64, dtype=torch.uint8, device="cuda"))
+    torch.cuda.synchronize()
+    assert torch.all(wide == 7.0)
+    sim.reset(wide[:, :20])  # the full width at row stride 24 is accepted and leaves the other columns alone
+    torch.cuda.synchronize()
+    assert torch.all(wide[:, 20:] == 7.0) and not torch.all(wide[:, :20] == 7.0)
     sim.close()
 
 

@@ -7,7 +7,6 @@ activations and tanh.approx; against an fp32 PyTorch forward of the same
 (pre-activations are O(1)); everything else (sampling algebra, GAE, running
 statistics, reward normalisation) is fp32/fp64 arithmetic compared at 1e-5.
 """
-import ctypes as C
 import math
 
 import numpy as np
@@ -220,7 +219,6 @@ def test_fused_statistics_forward_equals_the_two_launches(env, n, fused):
 def test_time_limit_bootstrap(env):
     """Envs that hover into the 402-step limit get reward += gamma * V(terminal_obs) (SB3 collect_rollouts)."""
     pkg, _lib, ppo = env
-    L = _lib.lib()
     thr = float(np.sqrt(0.1 * 9.81 / 4.0))
     n = 300
     cfg = pkg.default_config()
@@ -233,15 +231,13 @@ def test_time_limit_bootstrap(env):
     sim.reset(obs)
     a = torch.zeros(n, 4, device="cuda"); a[:, 3] = 2 * thr - 1
     a[::3, 3] = 1.0  # every third env rockets out of the dome instead (terminated, not truncated)
-    cnt, idx = C.c_void_p(), C.c_void_p()
-    assert L.qx_done_queue(sim._h, C.byref(cnt), C.byref(idx)) == 0
+    queue = sim.done_queue()
     seen_trunc = seen_term = 0
     for k in range(12):
-        assert L.qx_step_begin(sim._h, a.data_ptr(), obs.data_ptr(), 0, 20, rew.data_ptr(), te.data_ptr(), tr.data_ptr(), tobs.data_ptr(), None) == 0
+        sim.step_begin(a, obs, rew, te, tr, tobs)
         before = rew.clone()
-        assert L.ppo_bootstrap_truncated(C.byref(pol.struct), tobs.data_ptr(), 20, n, None, None, 0.0, cnt, idx, te.data_ptr(), tr.data_ptr(),
-                                         0.99, rew.data_ptr(), None) == 0
-        assert L.qx_step_end(sim._h, obs.data_ptr(), 0, 20, None) == 0
+        ppo.bootstrap_truncated(pol, tobs, None, 0.0, queue, te, tr, 0.99, rew)
+        sim.step_end(obs)
         torch.cuda.synchronize()
         trunc_only = tr.bool() & ~te.bool()
         with torch.no_grad():
@@ -256,13 +252,14 @@ def test_time_limit_bootstrap(env):
             st, acc = ppo.RunningStats(1, "cuda"), torch.zeros(n, device="cuda")
             st.stats[1] = 4.0  # a return variance that is not 1
             out, dn = torch.full((n,), 123.0, device="cuda"), torch.zeros(n, dtype=torch.uint8, device="cuda")
-            boot = (C.byref(pol.struct), tobs.data_ptr(), 20, n, None, None, 0.0, cnt, idx, te.data_ptr(), tr.data_ptr(), 0.99, out.data_ptr(), None)
-            nrm = (before.data_ptr(), te.data_ptr(), tr.data_ptr(), acc.data_ptr(), n, 0.99, 10.0, st.eps, st.stats.data_ptr(), out.data_ptr(), dn.data_ptr(),
-                   st.scratch.data_ptr(), None)
+            boot = (pol, tobs, None, 0.0, queue, te, tr, 0.99, out)
+            nrm = (before, te, tr, acc, st, 0.99, 10.0, out, dn)
             if first:
-                assert L.ppo_bootstrap_truncated_first(*boot) == 0 and L.ppo_reward_normalize_add(*nrm) == 0
+                ppo.bootstrap_truncated(*boot, first=True)
+                ppo.reward_normalize(*nrm, add=True)
             else:
-                assert L.ppo_reward_normalize(*nrm) == 0 and L.ppo_bootstrap_truncated(*boot) == 0
+                ppo.reward_normalize(*nrm)
+                ppo.bootstrap_truncated(*boot)
             torch.cuda.synchronize()
             outs.append((out.clone(), dn.clone(), acc.clone(), st.stats.clone()))
         assert (outs[0][0] - outs[1][0]).abs().max().item() < 1e-5 and torch.equal(outs[0][1], outs[1][1])

@@ -397,7 +397,7 @@ def test_invalid_arguments(pkg):
     sim = pkg.QuadXSim(64)
     buf = torch.empty(64, 128, 128, 4, dtype=torch.uint8, device=sim.device)
     idx = torch.zeros(4, dtype=torch.int32, device=sim.device)
-    s = sim._stream()
+    s = _lib.stream(sim.device)
     ptr = lambda t: C.c_void_p(t.data_ptr())  # noqa: E731
     cases = [
         (lambda: L.qx_render(sim._h, None, 64, 2, ptr(buf), s), "fmt is QX_FRAME_RGBA or QX_FRAME_MASK"),
