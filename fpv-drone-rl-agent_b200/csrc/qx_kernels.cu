@@ -1471,9 +1471,24 @@ static int launch(QxHandle* h, int mode, qx::StepArgs a, cudaStream_t s) {
   return QX_OK;
 }
 
+// The kernels access these buffers with vector instructions, which fault on a misaligned address: observation rows are
+// written as 16-byte (f32) / 8-byte (bf16) vectors when obs_stride is a multiple of 4 (write_obs; any other stride takes
+// the scalar stores), hover actions are read as one float4 per env and terminal-observation rows (stride obs_dim) are
+// written as float4.  A call that would issue such an access is refused before anything is launched.
+static bool misaligned(const void* p, uintptr_t bytes) { return p && reinterpret_cast<uintptr_t>(p) % bytes != 0; }
+static int check_alignment(const QxHandle* h, const char* fn, const float* actions_dev, const void* obs_dev, int32_t obs_dtype,
+                           int64_t obs_stride, const float* terminal_obs_dev) {
+  if (obs_stride % 4 == 0 && misaligned(obs_dev, obs_dtype == QX_OBS_BF16 ? 8 : 16))
+    return fail(QX_EINVAL, "%s: obs_dev must be 16-byte (f32) / 8-byte (bf16) aligned when obs_stride is a multiple of 4", fn);
+  if (h->dev.task == QX_TASK_HOVER && misaligned(actions_dev, 16)) return fail(QX_EINVAL, "%s: actions_dev must be 16-byte aligned", fn);
+  if (misaligned(terminal_obs_dev, 16)) return fail(QX_EINVAL, "%s: terminal_obs_dev must be 16-byte aligned", fn);
+  return QX_OK;
+}
+
 extern "C" int qx_reset(QxHandle* h, const uint8_t* mask_dev, void* obs_dev, int32_t obs_dtype, int64_t obs_stride, void* stream) {
   if (!h) return fail(QX_EINVAL, "qx_reset: null handle");
   if (obs_dev && obs_stride < h->dev.obs_dim) return fail(QX_EINVAL, "qx_reset: obs_stride < obs_dim");
+  if (int rc = check_alignment(h, "qx_reset", nullptr, obs_dev, obs_dtype, obs_stride, nullptr)) return rc;
   qx::StepArgs a{};
   a.state = h->state; a.mask = mask_dev; a.obs = obs_dev; a.obs_stride = obs_stride; a.obs_bf16 = obs_dtype == QX_OBS_BF16;
   a.stats = h->stats; a.n = h->n; a.k = 1;
@@ -1484,6 +1499,7 @@ extern "C" int qx_step_k(QxHandle* h, int32_t k, const float* actions_dev, float
                          uint8_t* terminated_dev, uint8_t* truncated_dev, void* stream) {
   if (!h || k <= 0 || !actions_dev || !reward_dev || !terminated_dev || !truncated_dev)
     return fail(QX_EINVAL, "qx_step_k: bad arguments");
+  if (int rc = check_alignment(h, "qx_step_k", actions_dev, obs_dev, QX_OBS_F32, h->dev.obs_dim, nullptr)) return rc;
   qx::StepArgs a{};
   a.state = h->state; a.actions = actions_dev; a.obs = obs_dev; a.obs_stride = h->dev.obs_dim; a.reward = reward_dev;
   a.terminated = terminated_dev; a.truncated = truncated_dev; a.stats = h->stats; a.n = h->n; a.k = k;
@@ -1494,6 +1510,7 @@ extern "C" int qx_step_begin(QxHandle* h, const float* actions_dev, void* obs_de
                              float* reward_dev, uint8_t* terminated_dev, uint8_t* truncated_dev, float* terminal_obs_dev, void* stream) {
   if (!h || !actions_dev || !reward_dev || !terminated_dev || !truncated_dev) return fail(QX_EINVAL, "qx_step: bad arguments");
   if (obs_dev && obs_stride < h->dev.obs_dim) return fail(QX_EINVAL, "qx_step: obs_stride < obs_dim");
+  if (int rc = check_alignment(h, "qx_step", actions_dev, obs_dev, obs_dtype, obs_stride, terminal_obs_dev)) return rc;
   qx::StepArgs a{};
   a.state = h->state; a.actions = actions_dev; a.obs = obs_dev; a.obs_stride = obs_stride; a.obs_bf16 = obs_dtype == QX_OBS_BF16;
   a.reward = reward_dev; a.terminated = terminated_dev; a.truncated = truncated_dev; a.terminal_obs = terminal_obs_dev;
@@ -1507,6 +1524,7 @@ extern "C" int qx_step_end(QxHandle* h, void* obs_dev, int32_t obs_dtype, int64_
   if (!h) return fail(QX_EINVAL, "qx_step_end: null handle");
   if (!h->cfg.auto_reset) return QX_OK;
   if (obs_dev && obs_stride < h->dev.obs_dim) return fail(QX_EINVAL, "qx_step_end: obs_stride < obs_dim");
+  if (int rc = check_alignment(h, "qx_step_end", nullptr, obs_dev, obs_dtype, obs_stride, nullptr)) return rc;
   if (use_merged(h)) return QX_OK;  // the step launch already re-created the finished envs
   qx::StepArgs a{};
   a.state = h->state; a.obs = obs_dev; a.obs_stride = obs_stride; a.obs_bf16 = obs_dtype == QX_OBS_BF16;
@@ -1523,6 +1541,7 @@ extern "C" int qx_step(QxHandle* h, const float* actions_dev, void* obs_dev, int
   if (h && h->cfg.auto_reset && h->n <= kInlineResetMaxEnvs && !(h->hot_mode == 1 && h->hot_ok)) {
     if (!actions_dev || !reward_dev || !terminated_dev || !truncated_dev) return fail(QX_EINVAL, "qx_step: bad arguments");
     if (obs_dev && obs_stride < h->dev.obs_dim) return fail(QX_EINVAL, "qx_step: obs_stride < obs_dim");
+    if (int rc = check_alignment(h, "qx_step", actions_dev, obs_dev, obs_dtype, obs_stride, terminal_obs_dev)) return rc;
     qx::StepArgs a{};
     a.state = h->state; a.actions = actions_dev; a.obs = obs_dev; a.obs_stride = obs_stride; a.obs_bf16 = obs_dtype == QX_OBS_BF16;
     a.reward = reward_dev; a.terminated = terminated_dev; a.truncated = truncated_dev; a.terminal_obs = terminal_obs_dev;

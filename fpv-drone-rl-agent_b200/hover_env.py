@@ -39,6 +39,14 @@ assert len(STATE_FIELDS) + len(CASCADE_FIELDS) == QX_STATE_WORDS_CASCADE
 _INT_FIELDS = {"step_count": np.int32, "rng_ctr": np.uint32, "flags": np.uint32}
 
 
+def _expect_aligned(t: torch.Tensor, name: str, nbytes: int) -> None:
+    """Raise ValueError naming `name` unless `t` starts on an `nbytes` boundary: the kernels access it with vector
+    instructions of that width (include/quadx_b200.h, Conventions), which fault on a misaligned address."""
+    if t.data_ptr() % nbytes:
+        raise ValueError(f"{name}: the kernels access this buffer with {nbytes}-byte vectors, so it must start on a {nbytes}-byte "
+                         f"boundary; got address {t.data_ptr():#x} (a column view such as buf[:, 1:21] is offset by its first column)")
+
+
 class Box:
     """Minimal stand-in for ``gymnasium.spaces.Box`` (hover.py:59-70)."""
 
@@ -98,6 +106,8 @@ class QuadXSim:
             raise ValueError("obs: expected [n_envs, >=obs_dim] with unit inner stride on the sim device")
         if obs.dtype not in (torch.float32, torch.bfloat16):
             raise TypeError("obs buffer must be float32 or bfloat16")
+        if obs.stride(0) % 4 == 0:  # rows written as 16-byte (f32) / 8-byte (bf16) vectors; other strides element by element
+            _expect_aligned(obs, "obs", 4 * obs.element_size())
         return obs.stride(0), QX_OBS_F32 if obs.dtype == torch.float32 else QX_OBS_BF16
 
     # -- device API ----------------------------------------------------------------
@@ -115,9 +125,12 @@ class QuadXSim:
         expect(reward, "reward", dtype=torch.float32, device=self.device, shape=(self.n,))
         expect(terminated, "terminated", dtype=torch.uint8, device=self.device, shape=(self.n,))
         expect(truncated, "truncated", dtype=torch.uint8, device=self.device, shape=(self.n,))
+        if self.act_dim == 4:
+            _expect_aligned(actions, "actions", 16)  # one float4 per env
         stride, code = self._obs_layout(obs)
         if terminal_obs is not None:
             expect(terminal_obs, "terminal_obs", dtype=torch.float32, device=self.device, shape=(self.n, self.obs_dim))
+            _expect_aligned(terminal_obs, "terminal_obs", 16)
         return (self._h, ptr(actions), ptr(obs), code, stride, ptr(reward), ptr(terminated), ptr(truncated), ptr(terminal_obs),
                 stream(self.device))
 
@@ -152,8 +165,11 @@ class QuadXSim:
                truncated: torch.Tensor) -> None:
         k = actions.shape[0]
         expect(actions, "actions", dtype=torch.float32, device=self.device, shape=(k, self.n, self.act_dim))
+        if self.act_dim == 4:
+            _expect_aligned(actions, "actions", 16)
         if obs is not None:
             expect(obs, "obs", dtype=torch.float32, device=self.device, shape=(k, self.n, self.obs_dim))
+            _expect_aligned(obs, "obs", 16)
         expect(reward, "reward", dtype=torch.float32, device=self.device, shape=(k, self.n))
         expect(terminated, "terminated", dtype=torch.uint8, device=self.device, shape=(k, self.n))
         expect(truncated, "truncated", dtype=torch.uint8, device=self.device, shape=(k, self.n))

@@ -16,6 +16,12 @@
  *   - pointers named *_host are ordinary host pointers; those calls copy
  *     through pinned staging buffers owned by the handle and return after the
  *     results are in host memory.
+ *   - device buffers of qx_reset / qx_step / qx_step_begin / qx_step_end / qx_step_k are accessed with vector
+ *     instructions and must be aligned accordingly, else the call returns QX_EINVAL and launches nothing:
+ *     obs_dev 16-byte (QX_OBS_F32) / 8-byte (QX_OBS_BF16) aligned when obs_stride is a multiple of 4 (any
+ *     other stride is written element by element, at any element-aligned address); hover actions_dev and
+ *     terminal_obs_dev 16-byte aligned.  cudaMalloc'd buffers and whole torch tensors are; a column view
+ *     such as buf[:, 1:21] of a [n, 24] f32 buffer is not.
  *   - a handle is not thread-safe; independent handles are.
  *   - one env == one drone in its own world (hover.py:78: one drone per Aviary).
  */

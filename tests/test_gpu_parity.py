@@ -23,7 +23,7 @@ import numpy as np
 import pytest
 import torch
 
-from tests.util import NONVISION_COLS, VISION_COLS, kernel_state_arrays, oracle_to_kernel_state
+from tests.util import NONVISION_COLS, VISION_COLS, ForkAccount, kernel_state_arrays, oracle_to_kernel_state
 
 pytestmark = pytest.mark.gpu
 
@@ -451,8 +451,7 @@ def test_batch_scale_parity_against_c_oracle(pkg, n):
     o2 = orc.reset().copy()
     _close(b.obs.cpu().numpy(), o2, 2e-3, "reset obs")
     rng = np.random.default_rng(5)
-    sync = np.ones(n, bool)
-    worst_obs, worst_rew, flips, seen, forked = 0.0, 0.0, 0, 0, 0
+    acc = ForkAccount(n)
     lift = rng.uniform(0, 1, n) < 0.7  # 70 % of the fleet lifts off, the rest idles into the floor rule of step 32
     for k in range(48):
         a = rng.uniform(-1, 1, (n, 4)).astype(np.float32)
@@ -460,29 +459,10 @@ def test_batch_scale_parity_against_c_oracle(pkg, n):
         a[:, 3] = np.where(lift, 0.2 + 0.1 * a[:, 3], -0.9)
         o, r, te, tr = b.step(sim, a)
         o2, r2, te2, tr2, _ = orc.step(a.astype(np.float64))
-        sync &= (te == te2) & (tr == tr2)
-        # a discontinuity of the model taken on different sides by fp32 and float64 (floor plane touched one sub-step
-        # earlier, motor saturation on / off) forks that env's trajectory for good: such envs are dropped like the ones
-        # whose flags differ, and COUNTED against the same budget
-        err = np.abs(o[:, NONVISION_COLS] - o2[:, NONVISION_COLS]).max(axis=1)
-        same_px = (o[:, 13] == o2[:, 13]) & (np.abs(o[:, 14] - o2[:, 14]) < 1e-4)
-        # (the yaw body rate enters the reward, hover.py:322-324, but not the observation: a fork can show there first)
-        fork = sync & ((err > 3e-3) | (same_px & (np.abs(r - r2) > 5e-3)))
-        forked += int(fork.sum())
-        sync &= ~fork
-        m = sync
-        worst_obs = max(worst_obs, float(err[m].max()))
-        same = m & same_px
-        flips += int((m & ~same).sum()); seen += int(m.sum())
-        worst_rew = max(worst_rew, float(np.abs(r[same] - r2[same]).max()))
-        # the flipped samples are not skipped: their reward error is bounded by one pixel row of the bbox ratio + visibility (0.45)
-        if (m & ~same).any():
-            assert float(np.abs(r[m & ~same] - r2[m & ~same]).max()) <= 2.5
-    print(f"n={n}: out-of-step envs {int((~sync).sum())} (of which forked at a discontinuity: {forked}), pixel-count flips {flips}/{seen}, "
-          f"worst obs err {worst_obs:.2e}, worst reward err {worst_rew:.2e}")
-    assert (~sync).sum() <= max(4, n // 500), int((~sync).sum())
-    assert flips <= 0.01 * seen, (flips, seen)
-    assert worst_obs <= 3e-3 and worst_rew <= 5e-3, (worst_obs, worst_rew)
+        acc.step(o, r, te, tr, o2, r2, te2, tr2)
+    print(f"n={n}: out-of-step envs {acc.out_of_step} (of which forked at a discontinuity: {acc.forked}), pixel-count flips {acc.flips}/{acc.seen}, "
+          f"worst obs err {acc.worst_obs:.2e}, worst reward err {acc.worst_rew:.2e}")
+    acc.check(max(4, n // 500))
     s1, s2 = sim.episode_stats(), orc.stats()
     assert abs(s1[2] - s2[2]) <= max(4, n // 500) and abs(s1[1] - s2[1]) <= 48 * max(4, n // 500)
     sim.close()

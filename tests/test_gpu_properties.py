@@ -269,40 +269,68 @@ def test_step_kernel_variants_are_bitwise_equal(pkg, monkeypatch):
     float2 = two envs per thread on packed FFMA2 / FMUL2 / FADD2, and S1 = one env per thread with its own components
     paired on the same packed instructions (csrc/qx_model.cuh, CoreS).  They are instantiated in the generic step kernel
     (any k, inline or queued reset), in the lean one-step kernel with a separate reset-queue launch, and in the merged
-    launch (the last resident wave of blocks drains the reset queue).  All perform the same IEEE operations per env, so
-    they must agree bit for bit -- states, observations, rewards, flags, episode statistics -- through
-    resets, for a batch size that leaves a thread with a single env, with the reference constants and with the generic
-    constants."""
+    launch (the last resident wave of blocks drains the reset queue); queued envs are re-created by the paired code or the
+    generic one (QX_PAIRED_RESET), in one of four launch shapes (QX_SHAPE), with or without programmatic dependent launches
+    (QX_PDL) and evict-first stores (QX_STREAM_STORES).  All perform the same IEEE operations per env, so they must agree
+    bit for bit -- states, observations, terminal observations, rewards, flags, episode statistics -- through resets, for a
+    batch size that leaves a thread with a single env, with the reference constants and with the generic constants.  The
+    done queue of every step is exact on every variant.  bf16 observations written into a stride-32 policy buffer through
+    the resets are the f32 ones rounded, on both reset paths."""
+    from tests.util import check_done_queue
+
     n, steps = 40000 + 77, 70
     g = torch.Generator(device="cuda").manual_seed(11)
     acts = (torch.rand(steps, n, 4, device="cuda", generator=g) * 2 - 1) * torch.tensor([0.5, 0.5, 0.5, 1.0], device="cuda")
     acts[..., 3] = acts[..., 3] * 0.4 + 0.05
+    paired4 = {"QX_HOT": "1", "QX_LANES": "4", "QX_MERGED": "0"}
     variants = [{"QX_HOT": "0"}, {"QX_HOT": "1", "QX_LANES": "1", "QX_MERGED": "1"}, {"QX_HOT": "1", "QX_LANES": "1", "QX_MERGED": "0"},
-                {"QX_HOT": "1", "QX_LANES": "4", "QX_MERGED": "1"}, {"QX_HOT": "1", "QX_LANES": "4", "QX_MERGED": "0"},
-                {"QX_HOT": "1", "QX_LANES": "2", "QX_MERGED": "1"}, {"QX_HOT": "1", "QX_LANES": "2", "QX_MERGED": "0"}]
+                {"QX_HOT": "1", "QX_LANES": "4", "QX_MERGED": "1"}, paired4,
+                {"QX_HOT": "1", "QX_LANES": "2", "QX_MERGED": "1"}, {"QX_HOT": "1", "QX_LANES": "2", "QX_MERGED": "0"},
+                {**paired4, "QX_MERGED": "1", "QX_PAIRED_RESET": "0"}, {**paired4, "QX_PAIRED_RESET": "0"},
+                {**paired4, "QX_SHAPE": "0"}, {**paired4, "QX_SHAPE": "3"}, {**paired4, "QX_SHAPE": "5"}, {**paired4, "QX_PDL": "0"},
+                {**paired4, "QX_STREAM_STORES": "1"}, {**paired4, "QX_STREAM_STORES": "2"}]
+    queue_lengths = set()
+
+    def run(var, bf16=False):
+        for k_ in ("QX_HOT", "QX_LANES", "QX_MERGED", "QX_PAIRED_RESET", "QX_SHAPE", "QX_PDL", "QX_STREAM_STORES"):
+            monkeypatch.delenv(k_, raising=False)
+        for k_, v_ in {"QX_LANES": "1", "QX_MERGED": "1", **var}.items():
+            monkeypatch.setenv(k_, v_)
+        sim = pkg.QuadXSim(n, pkg.default_config(), seed=5)  # floor start, idle steps, auto-reset, noise
+        d = sim.device
+        # bf16: the policy's input buffer, row stride 32; the kernels write the first 20 columns
+        obs = torch.zeros(steps, n, 32, device=d, dtype=torch.bfloat16)[..., :20] if bf16 else torch.zeros(steps, n, 20, device=d)
+        tobs = torch.zeros(steps, n, 20, device=d); rew = torch.zeros(steps, n, device=d)
+        te = torch.zeros(steps, n, dtype=torch.uint8, device=d); tr = torch.zeros(steps, n, dtype=torch.uint8, device=d)
+        o0 = torch.zeros(n, 20, device=d)
+        sim.reset(o0)
+        for k in range(steps):
+            sim.step_begin(acts[k], obs[k], rew[k], te[k], tr[k], tobs[k])
+            torch.cuda.synchronize()
+            queue_lengths.add(check_done_queue(sim, (te[k] | tr[k]).bool().cpu().numpy())[0])
+            sim.step_end(obs[k])
+        torch.cuda.synchronize()
+        out = (obs, tobs, rew, te, tr, sim.get_state(), sim.episode_stats())
+        sim.close()
+        return out
+
     for generic in (False, True):
         if generic:
             monkeypatch.setenv("QX_FORCE_GENERIC", "1")
-        out = []
-        for var in variants:
-            for k_, v_ in {"QX_LANES": "1", "QX_MERGED": "1", **var}.items():
-                monkeypatch.setenv(k_, v_)
-            sim = pkg.QuadXSim(n, pkg.default_config(), seed=5)  # floor start, idle steps, auto-reset, noise
-            d = sim.device
-            obs = torch.zeros(steps, n, 20, device=d); rew = torch.zeros(steps, n, device=d)
-            te = torch.zeros(steps, n, dtype=torch.uint8, device=d); tr = torch.zeros(steps, n, dtype=torch.uint8, device=d)
-            o0 = torch.zeros(n, 20, device=d)
-            sim.reset(o0)
-            for k in range(steps):
-                sim.step(acts[k], obs[k], rew[k], te[k], tr[k], split=True)
-            torch.cuda.synchronize()
-            out.append((obs, rew, te, tr, sim.get_state(), sim.episode_stats()))
-            sim.close()
-        o1, r1, te1, tr1, s1, e1 = out[0]
+        o1, t1, r1, te1, tr1, s1, e1 = run(variants[0])
         assert int(te1.sum()) > n // 2  # episodes ended (floor rule) and restarted
-        for vi, (o2, r2, te2, tr2, s2, e2) in enumerate(out[1:], 1):
-            assert torch.equal(te1, te2) and torch.equal(tr1, tr2) and e1[1:] == e2[1:], variants[vi]
-            assert torch.equal(o1.view(torch.int32), o2.view(torch.int32)), (variants[vi], float((o1 - o2).abs().max()))
-            assert torch.equal(r1.view(torch.int32), r2.view(torch.int32)), (variants[vi], float((r1 - r2).abs().max()))
+        for var in variants[1:]:
+            o2, t2, r2, te2, tr2, s2, e2 = run(var)
+            assert torch.equal(te1, te2) and torch.equal(tr1, tr2) and e1[1:] == e2[1:], var
+            assert torch.equal(o1.view(torch.int32), o2.view(torch.int32)), (var, float((o1 - o2).abs().max()))
+            assert torch.equal(t1.view(torch.int32), t2.view(torch.int32)), (var, float((t1 - t2).abs().max()))
+            assert torch.equal(r1.view(torch.int32), r2.view(torch.int32)), (var, float((r1 - r2).abs().max()))
             for k in s1:
-                assert np.array_equal(s1[k].view(np.uint32), s2[k].view(np.uint32)), (variants[vi], k)
+                assert np.array_equal(s1[k].view(np.uint32), s2[k].view(np.uint32)), (var, k)
+            del o2, t2
+        for var in (paired4, {**paired4, "QX_PAIRED_RESET": "0"}):
+            ob = run(var, bf16=True)[0]
+            assert torch.equal(ob.view(torch.int16), o1.to(torch.bfloat16).view(torch.int16)), var
+            assert torch.all(ob.as_strided((steps, n, 12), (n * 32, 32, 1), 20) == 0), var
+    print(f"done-queue lengths seen over the variants: {len(queue_lengths)} distinct, max {max(queue_lengths)} of {n} envs")
+    assert 0 in queue_lengths and len(queue_lengths) > 3
