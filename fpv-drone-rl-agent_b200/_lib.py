@@ -67,6 +67,13 @@ class PpoPolicy(C.Structure):
                 ("b2", C.c_void_p), ("b3", C.c_void_p), ("log_std", C.c_void_p), ("obs_dim", i32), ("act_dim", i32)]
 
 
+class SacActor(C.Structure):
+    """Mirror of ``struct SacActor`` in include/sac_b200.h."""
+
+    _fields_ = [("w1", C.c_void_p), ("w2", C.c_void_p), ("w_mu", C.c_void_p), ("b1", C.c_void_p), ("b2", C.c_void_p), ("b_mu", C.c_void_p),
+                ("obs_dim", i32), ("act_dim", i32)]
+
+
 _lib = None
 
 
@@ -137,6 +144,8 @@ def lib() -> C.CDLL:
         "ppo_update_kl_stop": (C.c_int, [vp, C.c_float, C.POINTER(i32), C.POINTER(i32), vp]),
         "ppo_update_set_log_std_floor": (C.c_int, [vp, i32, C.c_float, vp]),
         "qx_debug_clock_probe": (C.c_int, [vp, vp]),
+        # include/sac_b200.h
+        "sac_actor_forward": (C.c_int, [C.POINTER(SacActor), vp, i64, i64, vp, vp, f32, vp, vp, vp]),
     }
     for name, (res, args) in protos.items():
         fn = getattr(L, name)  # AttributeError here = header and library disagree
@@ -155,6 +164,8 @@ EXPORTED = [
 PPO_EXPORTED = ["ppo_policy_forward", "ppo_policy_forward_stats", "ppo_bootstrap_truncated", "ppo_bootstrap_truncated_first", "ppo_reward_normalize_add", "ppo_gae", "ppo_running_stats_update", "ppo_running_stats_scratch_bytes",
                 "ppo_reward_normalize", "ppo_test_gemm", "ppo_test_gemm_mn", "ppo_test_tanh_bf16", "ppo_update_num_params", "ppo_update_workspace_bytes",
                 "ppo_update_minibatch", "ppo_update_grad_norm", "ppo_update_adam", "ppo_update_step_count", "ppo_update_set_lr_scale", "ppo_update_kl_stop", "ppo_update_set_log_std_floor", "ppo_update_recompute_logp"]
+
+SAC_EXPORTED = ["sac_actor_forward"]
 
 
 class QxError(RuntimeError):

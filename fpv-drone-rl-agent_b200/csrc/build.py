@@ -13,8 +13,9 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 LIB = os.environ.get("QX_LIB_OUT") or os.path.join(HERE, "libquadx_b200.so")  # QX_LIB_OUT: tuning builds (QX_NVCC_EXTRA) next to the product library
-SOURCES = ["qx_kernels.cu", "ppo_kernels.cu", "ppo_update_kernels.cu"]
-HEADERS = ["qx_model.cuh", "qx_lanes.cuh", "qx_ref_constants.cuh", "qx_internal.h", "tc05.cuh", os.path.join(ROOT, "include", "quadx_b200.h"), os.path.join(ROOT, "include", "ppo_b200.h")]
+SOURCES = ["qx_kernels.cu", "ppo_kernels.cu", "ppo_update_kernels.cu", "sac_kernels.cu"]
+HEADERS = ["qx_model.cuh", "qx_lanes.cuh", "qx_ref_constants.cuh", "qx_internal.h", "tc05.cuh", os.path.join(ROOT, "include", "quadx_b200.h"), os.path.join(ROOT, "include", "ppo_b200.h"),
+           os.path.join(ROOT, "include", "sac_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17", "--use_fast_math",  # FTZ + approximate div/sqrt in the once-per-step epilogue; parity tests hold

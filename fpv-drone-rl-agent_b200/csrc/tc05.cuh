@@ -117,4 +117,43 @@ __device__ __forceinline__ void stage_weight(uint8_t* smem, const __nv_bfloat16*
   }
 }
 
+// ---- the slot scheme of the persistent MLP kernels -----------------------------------------------------------------
+// A CTA runs several independent "slots" (groups of consecutive warps), each walking its own sequence of 128-row tiles, so
+// that one slot's epilogue overlaps another slot's tcgen05.mma chain.  A slot synchronises on its own named barrier
+// (id slot + 1; id 0 is __syncthreads).
+__device__ __forceinline__ void slot_barrier(int slot, uint32_t slot_threads) {
+  asm volatile("bar.sync %0, %1;" ::"r"(slot + 1), "r"(slot_threads) : "memory");
+}
+
+// Slot-major tile order: tile t belongs to CTA t % grid, so the tiles that do not fill a whole round of grid x slots are
+// spread over the CTAs instead of giving the first CTAs a tile in every slot.  Slot `slot` of CTA `cta` starts at the
+// returned tile and steps by grid * slots.
+__device__ __forceinline__ int slot_major_first_tile(int slot, int cta, int grid) { return slot * grid + cta; }
+
+// Row `src[0 .. cols)` of an fp32 matrix -> x[0 .. cols), zeros beyond.  vec: src is 16-byte aligned (base pointer and row
+// stride decided once per launch on the host, so the branch is uniform): float4 loads where four columns fit, scalar ones
+// elsewhere.
+template <int N>
+__device__ __forceinline__ void load_f32_row(const float* __restrict__ src, int cols, bool vec, float (&x)[N]) {
+  static_assert(N % 4 == 0, "whole float4 groups");
+#pragma unroll
+  for (int j = 0; j < N; ++j) x[j] = 0.f;
+  if (vec) {
+#pragma unroll
+    for (int v = 0; v < N / 4; ++v)
+      if (4 * v + 4 <= cols) {
+        const float4 t = __ldg(reinterpret_cast<const float4*>(src + 4 * v));
+        x[4 * v] = t.x; x[4 * v + 1] = t.y; x[4 * v + 2] = t.z; x[4 * v + 3] = t.w;
+      } else {
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+          if (4 * v + j < cols) x[4 * v + j] = __ldg(src + 4 * v + j);
+      }
+  } else {
+#pragma unroll
+    for (int j = 0; j < N; ++j)
+      if (j < cols) x[j] = __ldg(src + j);
+  }
+}
+
 }  // namespace tc05

@@ -213,6 +213,11 @@ class PackedPolicy:
         self.b3[ad].copy_(m.v.bias[0])
         self.log_std[:ad].copy_(m.log_std)
 
+    def act(self, obs: torch.Tensor, env_actions: torch.Tensor, norm: tuple | None, obs_clip: float) -> None:
+        """The deterministic action of one playback step (``model.predict(obs, deterministic=True)``): the action mean clipped to
+        the action box, into env_actions.  The counterpart of ``sac.PackedSacActor.act``, so that PolicyEvaluator serves both."""
+        policy_forward(self, obs, norm=norm, obs_clip=obs_clip, deterministic=True, env_actions=env_actions)
+
 
 class RunningStats:
     """VecNormalize ``RunningMeanStd`` kept on the device: {mean[dim], var[dim], count} in fp64."""
@@ -301,9 +306,12 @@ class PolicyEvaluator:
     A chunk of ``chunk`` such steps is one CUDA-graph replay (``use_cuda_graph=False``: eager launches, same results); the host
     reads the number of closed records once per chunk.  Every ``evaluate()`` starts from the state the first reset produced,
     motor-noise counters included, so two evaluations of the same policy give the same numbers.  The packed policy is read
-    where it lives: an evaluator built once follows the weights of a policy that keeps training."""
+    where it lives: an evaluator built once follows the weights of a policy that keeps training.
 
-    def __init__(self, policy: PackedPolicy, obs_stats: RunningStats | None, env_cfg=None, n_episodes: int = 4096, seed: int = 0,
+    ``policy`` is a ``PackedPolicy`` (PPO) or a ``sac.PackedSacActor`` (an imported SB3 SAC actor, ``sac.load_sb3_zip``): the
+    evaluator only calls its ``act(obs, env_actions, norm, obs_clip)``."""
+
+    def __init__(self, policy: "PackedPolicy | sac.PackedSacActor", obs_stats: RunningStats | None, env_cfg=None, n_episodes: int = 4096, seed: int = 0,
                  task: int = 0, obs_clip: float = 10.0, device=None, chunk: int = 32, use_cuda_graph: bool = True):
         if n_episodes <= 0 or chunk <= 0:
             raise ValueError("n_episodes and chunk must be positive")
@@ -338,11 +346,11 @@ class PolicyEvaluator:
         self._state0 = self.sim.get_state()
         self._graph = None
         # one-time kernel attribute setup must not happen inside a graph capture
-        policy_forward(self.pol, self.obs, norm=self.norm, obs_clip=self.obs_clip, deterministic=True, env_actions=self.env_actions)
+        self.pol.act(self.obs, self.env_actions, self.norm, self.obs_clip)
 
     def _chunk(self) -> None:
         for _ in range(self.chunk):
-            policy_forward(self.pol, self.obs, norm=self.norm, obs_clip=self.obs_clip, deterministic=True, env_actions=self.env_actions)
+            self.pol.act(self.obs, self.env_actions, self.norm, self.obs_clip)
             self.sim.step(self.env_actions, self.obs, self.reward, self.te, self.tr)
             self.sim.episode_record(self.ret, self.length, self.end, self.n_closed)
 
@@ -389,7 +397,7 @@ class PolicyEvaluator:
         self.sim.close()
 
 
-def evaluate_policy(policy: PackedPolicy, obs_stats: RunningStats | None, env_cfg=None, n_episodes: int = 4096, seed: int = 0,
+def evaluate_policy(policy: "PackedPolicy | sac.PackedSacActor", obs_stats: RunningStats | None, env_cfg=None, n_episodes: int = 4096, seed: int = 0,
                     task: int = 0, obs_clip: float = 10.0, device=None, **kw) -> tuple[dict, dict]:
     """One evaluation with a PolicyEvaluator built for it (kw: chunk, use_cuda_graph); (summary, records) as evaluate()."""
     ev = PolicyEvaluator(policy, obs_stats, env_cfg, n_episodes, seed, task, obs_clip, device, **kw)
